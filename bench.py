@@ -1,7 +1,14 @@
 #!/usr/bin/env python
 """bench.py — env-steps/sec of the batched Pommerman step path on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what its timed region computed as .npy files, so that two builds
+can be compared output for output (the inputs depend only on the arguments):
+  status.npy  float32 [n_envs]              status byte of every env after the last timed step
+  states.npy  float64 [DUMP_ENVS, 263]      the full State of a fixed, seeded sample of envs after the last timed step,
+                                            every field of include/pom_state.h flattened in declaration order
+  stats.npy   float64 [10]                  the episode counters of the warmup + timed steps (pom_batch_stats)
 
 Own arm (default): BASELINE.json configs[2] — 1,048,576 envs per GPU, random joint actions incl. bombs,
 kicks and chain explosions, PER-TICK kernel (pom_batch_step, auto-reset on so every env is live on every
@@ -60,6 +67,7 @@ ROLLOUT_TICKS = 800
 EXPAND_ROOTS, EXPAND_FANOUT = 4096, 1296
 STRONG_TOTAL = 1 << 20
 PARITY_ENVS, PARITY_TICKS = 64, 48
+DUMP_ENVS = 16384            # --dump-outputs: 16 Ki sampled States, 34 MB as float64
 
 
 def measured_peak():
@@ -294,6 +302,20 @@ def oracle_replay(O, T, first_env, global_envs, ticks, seed, max_ticks):
     return np.concatenate(out_S), np.concatenate(out_st)
 
 
+def dump_outputs(pb, b, counters, out_dir):
+    """--dump-outputs: the timed region's results on `b` (see the module docstring); call before anything else steps `b`"""
+    from numpy.lib import recfunctions
+    idx = np.sort(np.random.default_rng(RNG_SEED).choice(b.n, min(DUMP_ENVS, b.n), replace=False)).astype(np.uint32)
+    small = pb.Batch(idx.shape[0], device=b.device, n_templates=1, empty=True)
+    small.clone_from(b, idx)
+    S, _ = small.download()
+    small.close()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "status.npy"), b.status().astype(np.float32))
+    np.save(os.path.join(out_dir, "states.npy"), recfunctions.structured_to_unstructured(S, dtype=np.float64))
+    np.save(os.path.join(out_dir, "stats.npy"), counters.astype(np.float64))
+
+
 def run_own(args):
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -361,6 +383,8 @@ def run_own(args):
     stats = b.stats()
     assert stats.env_steps == n * (K + W), "kernel did not step every env on every tick"
     counters_main = b.stats().as_array()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(pb, b, counters_main, args.dump_outputs)
     flags &= ~pb.STEP_OVERLAP
 
     # ---- e2e: HOST buffers through the C ABI, every tick, the host waits for every result.  The envs run as two
@@ -669,7 +693,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="own", choices=["own", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed region's results to DIR/*.npy (own arm; with several GPUs, rank 0's shard)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "own":
+        ap.error("--dump-outputs applies to the own arm")
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
