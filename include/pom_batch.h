@@ -86,15 +86,21 @@ typedef struct pom_init_desc {
 } pom_init_desc;
 
 enum {
-    POM_INIT_EMPTY = 0x1   /* do not fill the envs (they will be uploaded); the pool is still built */
+    POM_INIT_EMPTY = 0x1,  /* do not fill the envs (they will be uploaded); the pool is still built */
+    POM_INIT_TEAMS = 0x2   /* the handle plays the 2v2 TEAM game: team 0 = agents 0 and 2, team 1 = agents 1 and 3.
+                              Step (bboard::Step) is the same, flames kill teammates too; what changes is when an episode
+                              ends and who won (pom_state.h: the status byte) and whom the device SimpleAgent treats as an
+                              enemy (not its teammate).  The reference has no team mode: this is the project's definition.
+                              The mode is fixed for the handle's life and applies to every entry point that steps or acts;
+                              pom_batch_clone / pom_batch_expand_step between handles of different modes fail (POM_E_ARG). */
 };
 
 /* episode counters accumulated on the device (Environment::IsDone/IsDraw/GetWinner, bboard.hpp:617-631) */
 typedef struct pom_stats {
     uint64_t env_steps;        /* Steps executed (finished/frozen envs not counted) */
     uint64_t episodes;         /* episodes finished (won + draw + truncated + invalid) */
-    uint64_t wins[4];          /* episodes won by agent 0..3                         */
-    uint64_t draws;            /* aliveAgents == 0                                   */
+    uint64_t wins[4];          /* episodes won by agent 0..3; team game: wins[t] by team t, wins[2] = wins[3] = 0 */
+    uint64_t draws;            /* aliveAgents == 0; team game: both teams out in the same tick */
     uint64_t truncated;        /* timeStep reached max_ticks                         */
     uint64_t sum_episode_len;  /* sum of timeStep over finished episodes             */
     uint64_t invalid;          /* episodes aborted because the env left the reference's defined domain
@@ -108,6 +114,8 @@ int  pom_batch_init(pom_batch** out, int device, uint64_t n_envs, const pom_init
 int  pom_batch_destroy(pom_batch* b);
 int  pom_batch_sync(pom_batch* b);
 const char* pom_last_error(void);
+/* 1 if the handle plays the team game (POM_INIT_TEAMS), 0 for free-for-all, POM_E_ARG for a null handle */
+int  pom_batch_teams(const pom_batch* b);
 
 /* ---- AoS <-> packed exchange (there is no reference call: State is passed by pointer) ---- */
 int  pom_batch_upload(pom_batch* b, uint64_t first, uint64_t count, const pom_state* states, const uint8_t* status /* may be NULL */);

@@ -237,8 +237,9 @@ private:
 class BatchEnvironment
 {
 public:
+    /* teams: the games are 2v2 team games (POM_INIT_TEAMS, include/pom_batch.h: agents 0 and 2 against 1 and 3) */
     BatchEnvironment(size_t nGames, int device = 0, uint64_t envOffset = 0, uint32_t nTemplates = 1024,
-                     int firstSeed = 0x1337, uint32_t maxTicks = 0);
+                     int firstSeed = 0x1337, uint32_t maxTicks = 0, bool teams = false);
     ~BatchEnvironment();
     BatchEnvironment(const BatchEnvironment&) = delete;
     BatchEnvironment& operator=(const BatchEnvironment&) = delete;
@@ -273,7 +274,9 @@ public:
     const std::vector<uint8_t>& Status();          /* POM_STATUS_* per game */
     bool IsDone(size_t i);
     bool IsDraw(size_t i);
-    int GetWinner(size_t i);
+    int GetWinner(size_t i);                       /* the winning agent; -1 while running, on a draw and in a team game */
+    bool IsTeamGame() const { return teams; }
+    int GetWinningTeam(size_t i);                  /* team game: the winning team (0 or 1); -1 while running, on a draw */
     pom_batch* Handle() const { return handle; }
 
 private:
@@ -286,6 +289,7 @@ private:
     bool fresh = false;
     uint32_t tick = 0;
     int viewRange = -1;
+    bool teams = false;
 };
 
 }

@@ -27,7 +27,7 @@ def ROLL_SIMPLE(agent_mask):
     return (agent_mask & 0xF) << 8
 
 
-INIT_EMPTY = 1
+INIT_EMPTY, INIT_TEAMS = 1, 2
 
 STATUS_DONE, STATUS_DRAW, STATUS_INVALID, STATUS_TRUNCATED = 0x01, 0x02, 0x10, 0x20
 
@@ -132,6 +132,7 @@ def lib():
         L.pom_rng_moves.argtypes = [u64, u64, u32, u32]
         L.pom_batch_generate_moves.argtypes = [vp, vp, u64, u32, u32]
         L.pom_batch_size.restype = u64
+        L.pom_batch_teams.argtypes = [vp]
         L.pom_batch_size.argtypes = [vp]
         L.pom_batch_device.argtypes = [vp]
         for f in ("pom_batch_stream", "pom_batch_stats_device_ptr", "pom_batch_records_device_ptr"):
@@ -171,13 +172,13 @@ class Batch:
     """One handle = one shard of envs on one GPU (pom_batch_* of include/pom_batch.h)."""
 
     def __init__(self, n_envs, device=0, env_offset=0, n_templates=1024, first_seed=0x1337,
-                 host_templates=None, max_ticks=0, empty=False):
+                 host_templates=None, max_ticks=0, empty=False, teams=False):
         self.h = C.c_void_p()
         d = InitDesc()
         d.env_offset = env_offset
         d.first_seed = first_seed
         d.max_ticks = max_ticks
-        d.flags = INIT_EMPTY if empty else 0
+        d.flags = (INIT_EMPTY if empty else 0) | (INIT_TEAMS if teams else 0)
         self._keep = None
         if host_templates is not None:
             assert host_templates.dtype == STATE_DT
@@ -204,6 +205,12 @@ class Batch:
             pass
 
     def sync(self): _ck(lib().pom_batch_sync(self.h))
+
+    def teams(self):
+        """True if the handle plays the 2v2 team game (pom_batch_teams)"""
+        r = lib().pom_batch_teams(self.h)
+        _ck(min(r, 0))
+        return r == 1
     def reset(self): _ck(lib().pom_batch_reset(self.h))
 
     def upload(self, states, status=None, first=0):

@@ -68,6 +68,8 @@ struct pom_batch {
     int       obs_fused = 0;                   /* POM_OBS_FUSED=1: pom_batch_step_observe / pom_step_compact_io::obs_dev write the planes
                                                   from inside the step kernel instead of launching k_observe_planes behind it */
     int       step_kernel = 0;                 /* 0 = k_step_ws (persistent, warp-specialised), 1 = k_step (one CTA per tile); POM_STEP_KERNEL=tile */
+    bool      teams = false;                   /* POM_INIT_TEAMS: the 2v2 team game, fixed for the handle's life; every stepping or
+                                                  acting launch takes the kernel images of this mode (POM_DISPATCH_MODE) */
     uint8_t*  recs = nullptr;
     uint8_t*  templates = nullptr;
     uint32_t* episodes = nullptr;
@@ -130,6 +132,8 @@ int use(const pom_batch* cb, bool join = true)
 /* The dynamic shared-memory limit of a kernel is a per-device attribute: remember it per handle (one handle = one
  * device), not in a process-wide flag, so that handles on other GPUs and other host threads set it for themselves. */
 enum { ATTR_STEP = 1, ATTR_ROLLOUT = 2, ATTR_ROLLOUT_POLICY = 4, ATTR_POLICY_MOVES = 8, ATTR_EXPAND = 16, ATTR_OBS = 32, ATTR_ROLLOUT_SPEC = 64, ATTR_OBS_CROPPED = 128 };
+/* the bit of a kernel's team image */
+constexpr uint32_t attr_bit(uint32_t which, bool teams) { return teams ? which << 8 : which; }
 
 template<typename K>
 int set_smem(pom_batch* b, uint32_t which, K kernel, uint32_t bytes)
@@ -234,19 +238,21 @@ int pack_into(pom_batch* b, uint8_t* dst_recs, uint64_t first, uint64_t count, c
 /* geometry of the persistent per-tick kernel (k_step_ws): compute warps and slice buffers per CTA (= per SM) */
 constexpr int WS_NW = 20, WS_NBUF = 24;
 
-template<int NW, bool OBS, bool FREEZE = false, bool SPEC = false>
+template<int NW, bool OBS, bool FREEZE = false, bool SPEC = false, bool TEAMS = false>
 int launch_step_ws(pom_batch* b, const pomk::BatchParams& P, const pomk::StepIO& io, uint32_t flags, cudaStream_t on)
 {
     typedef pomk::RingScratch<WS_NBUF> R;
-    const uint32_t bit = SPEC ? 2u : (FREEZE ? 1u : (1u << (NW + (OBS ? 1 : 0))));    /* NW is even and >= 12 */
+    /* NW is even and >= 12; the team images (NW = WS_NW only) take bits 24..26 */
+    const uint32_t bit = TEAMS ? (1u << (24 + (FREEZE ? 2 : (OBS ? 1 : 0)))) :
+                         SPEC ? 2u : (FREEZE ? 1u : (1u << (NW + (OBS ? 1 : 0))));
     if(!(b->attr_ws & bit))
     {
-        CK(cudaFuncSetAttribute(pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(R::BYTES)));
+        CK(cudaFuncSetAttribute(pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC, TEAMS>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(R::BYTES)));
         b->attr_ws |= bit;
     }
     const uint64_t n_slices = (P.n_envs + 31) / 32;
     const unsigned grid = unsigned(n_slices < uint64_t(b->n_sms) ? n_slices : uint64_t(b->n_sms));
-    pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC><<<grid, (NW + 1) * 32, R::BYTES, on ? on : b->stream>>>(P, io, flags);
+    pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC, TEAMS><<<grid, (NW + 1) * 32, R::BYTES, on ? on : b->stream>>>(P, io, flags);
     b->launches++;
     CK(cudaGetLastError());
     return POM_OK;
@@ -257,6 +263,13 @@ int launch_step_io(pom_batch* b, const pomk::BatchParams& P, pomk::StepIO io, ui
     io.bulk = (reinterpret_cast<uintptr_t>(io.moves) & 15u) == 0u ? 1u : 0u;   /* TMA needs 16-byte alignment */
     /* whole-batch launches alternate the direction of the walk (L2 reuse between ticks, see StepIO::reverse) */
     if(P.n_envs == b->n_envs && b->pingpong) io.reverse = (b->walk++) & 1u;
+    if(b->teams)
+    {
+        /* the team game has the generic images of the default geometry only: no SPEC image, no POM_WS_NW variants */
+        if(flags & pomk::STEP_FREEZE_TRUNCATED) return launch_step_ws<WS_NW, false, true, false, true>(b, P, io, flags, on);
+        if(io.obs) return launch_step_ws<WS_NW, true, false, false, true>(b, P, io, flags, on);
+        return launch_step_ws<WS_NW, false, false, false, true>(b, P, io, flags, on);
+    }
     if(flags & pomk::STEP_FREEZE_TRUNCATED) return launch_step_ws<WS_NW, false, true>(b, P, io, flags, on);
     /* the specialised image (k_step_ws, SPEC) for the plain loop */
     if(b->ws_nw == WS_NW && (flags & ~uint32_t(POM_STEP_OVERLAP)) == uint32_t(POM_STEP_AUTORESET | POM_STEP_COUNT) && io.bulk &&
@@ -275,7 +288,7 @@ int launch_step_io(pom_batch* b, const pomk::BatchParams& P, pomk::StepIO io, ui
     }
 }
 
-template<int TPB>
+template<int TPB, bool TEAMS = false>
 int launch_step(pom_batch* b, const uint8_t* moves_dev, uint32_t flags, uint8_t* status_dev, uint64_t first = 0, uint64_t count = 0, cudaStream_t on = nullptr,
                 bool tile_kernel = false)
 {
@@ -294,15 +307,15 @@ int launch_step(pom_batch* b, const uint8_t* moves_dev, uint32_t flags, uint8_t*
         io.status_out = status_dev;
         return launch_step_io(b, P, io, flags, on);
     }
-    { int rc = set_smem(b, ATTR_STEP, pomk::k_step<TPB>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc; }
+    { int rc = set_smem(b, attr_bit(ATTR_STEP, TEAMS), pomk::k_step<TPB, TEAMS>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc; }
     const unsigned grid = unsigned((P.n_envs + TPB - 1) / TPB);
-    pomk::k_step<TPB><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, on ? on : b->stream>>>(P, reinterpret_cast<const uint32_t*>(moves_dev), flags, status_dev);
+    pomk::k_step<TPB, TEAMS><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, on ? on : b->stream>>>(P, reinterpret_cast<const uint32_t*>(moves_dev), flags, status_dev);
     b->launches++;
     CK(cudaGetLastError());
     return POM_OK;
 }
 
-template<int TPB>
+template<int TPB, bool TEAMS = false>
 int launch_rollout(pom_batch* b, uint32_t ticks, uint64_t seed, uint32_t tick0, uint32_t flags, const uint8_t* move_seq = nullptr)
 {
     const uint32_t n_actions = (flags & POM_ROLL_HARMLESS) ? 5u : 6u, no_reset = flags & (POM_ROLL_NO_RESET | POM_ROLL_CONTINUE_UNDEFINED);
@@ -310,31 +323,31 @@ int launch_rollout(pom_batch* b, uint32_t ticks, uint64_t seed, uint32_t tick0, 
     const unsigned grid = unsigned((b->n_envs + TPB - 1) / TPB);
     if(mask)
     {
-        int rc = set_smem(b, ATTR_ROLLOUT_POLICY, pomk::k_rollout<TPB, true>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
+        int rc = set_smem(b, attr_bit(ATTR_ROLLOUT_POLICY, TEAMS), pomk::k_rollout<TPB, true, false, TEAMS>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
         rc = ensure_policy(b); if(rc) return rc;
-        pomk::k_rollout<TPB, true><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), ticks, seed, tick0, n_actions, no_reset, mask, nullptr);
+        pomk::k_rollout<TPB, true, false, TEAMS><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), ticks, seed, tick0, n_actions, no_reset, mask, nullptr);
     }
-    else if(n_actions == 6u && no_reset == 0u && !move_seq && !b->no_spec)
+    else if(!TEAMS && n_actions == 6u && no_reset == 0u && !move_seq && !b->no_spec)      /* the SPEC image is free-for-all only */
     {
         int rc = set_smem(b, ATTR_ROLLOUT_SPEC, pomk::k_rollout<TPB, false, true>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
         pomk::k_rollout<TPB, false, true><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), ticks, seed, tick0, 6u, 0u, 0u, nullptr);
     }
     else
     {
-        int rc = set_smem(b, ATTR_ROLLOUT, pomk::k_rollout<TPB, false>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
-        pomk::k_rollout<TPB, false><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), ticks, seed, tick0, n_actions, no_reset, 0u, reinterpret_cast<const uint32_t*>(move_seq));
+        int rc = set_smem(b, attr_bit(ATTR_ROLLOUT, TEAMS), pomk::k_rollout<TPB, false, false, TEAMS>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
+        pomk::k_rollout<TPB, false, false, TEAMS><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), ticks, seed, tick0, n_actions, no_reset, 0u, reinterpret_cast<const uint32_t*>(move_seq));
     }
     b->launches++;
     CK(cudaGetLastError());
     return POM_OK;
 }
 
-template<int TPB>
+template<int TPB, bool TEAMS = false>
 int launch_policy_moves(pom_batch* b, uint8_t* moves_dev, uint64_t seed, uint32_t tick, uint32_t mask, uint32_t gen_actions = 0, uint32_t freeze_truncated = 0)
 {
-    { int rc = set_smem(b, ATTR_POLICY_MOVES, pomk::k_policy_moves<TPB>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc; }
+    { int rc = set_smem(b, attr_bit(ATTR_POLICY_MOVES, TEAMS), pomk::k_policy_moves<TPB, TEAMS>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc; }
     const unsigned grid = unsigned((b->n_envs + TPB - 1) / TPB);
-    pomk::k_policy_moves<TPB><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), reinterpret_cast<uint32_t*>(moves_dev), seed, tick, mask, gen_actions, freeze_truncated);
+    pomk::k_policy_moves<TPB, TEAMS><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), reinterpret_cast<uint32_t*>(moves_dev), seed, tick, mask, gen_actions, freeze_truncated);
     b->launches++;
     CK(cudaGetLastError());
     return POM_OK;
@@ -361,12 +374,12 @@ int launch_observe_planes(pom_batch* b, uint8_t* obs_dev, uint32_t mask, int vie
     return POM_OK;
 }
 
-template<int TPB>
+template<int TPB, bool TEAMS = false>
 int launch_expand(pom_batch* dst, const pom_batch* src, const uint32_t* idx_dev, uint64_t n_children, uint32_t fanout, uint32_t flags)
 {
-    { int rc = set_smem(dst, ATTR_EXPAND, pomk::k_expand_step<TPB>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc; }
+    { int rc = set_smem(dst, attr_bit(ATTR_EXPAND, TEAMS), pomk::k_expand_step<TPB, TEAMS>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc; }
     const unsigned grid = unsigned((n_children + TPB - 1) / TPB);
-    pomk::k_expand_step<TPB><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, dst->stream>>>(dst->recs, src->recs, idx_dev, n_children, fanout, flags);
+    pomk::k_expand_step<TPB, TEAMS><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, dst->stream>>>(dst->recs, src->recs, idx_dev, n_children, fanout, flags);
     dst->launches++;
     CK(cudaGetLastError());
     return POM_OK;
@@ -427,6 +440,13 @@ bool local_cpus(int device, cpu_set_t* set)
         if((h)->tpb == 256) return fn<256>(__VA_ARGS__); \
         return fn<128>(__VA_ARGS__); \
     } while(0)
+/* the same for the launches that step or act: a team handle takes the team images, which exist for the default
+ * geometry only (POM_TPB does not apply to it) */
+#define POM_DISPATCH_MODE(h, fn, ...) \
+    do { \
+        if((h)->teams) return fn<128, true>(__VA_ARGS__); \
+        POM_DISPATCH(h, fn, __VA_ARGS__); \
+    } while(0)
 
 extern "C" {
 
@@ -456,6 +476,7 @@ int pom_batch_init(pom_batch** out, int device, uint64_t n_envs, const pom_init_
     b->env_offset = desc->env_offset;
     b->n_templates = desc->n_templates;
     b->max_ticks = desc->max_ticks;
+    b->teams = (desc->flags & POM_INIT_TEAMS) != 0;
     cudaDeviceGetAttribute(&b->n_sms, cudaDevAttrMultiProcessorCount, device);
     if(b->n_sms < 1) b->n_sms = 1;
     if(const char* e = std::getenv("POM_STEP_KERNEL")) b->step_kernel = std::strcmp(e, "tile") == 0 ? 1 : 0;
@@ -648,7 +669,7 @@ int pom_batch_step(pom_batch* b, const uint8_t* moves_dev, uint32_t flags)
     const bool overlap = (flags & POM_STEP_OVERLAP) && b && b->n_envs >= (uint64_t(1) << 18);
     int rc = use(b, !overlap); if(rc) return rc;
     if(!moves_dev) return fail(POM_E_ARG, "pom_batch_step: null moves");
-    if(!overlap) POM_DISPATCH(b, launch_step, b, moves_dev, flags, nullptr);
+    if(!overlap) POM_DISPATCH_MODE(b, launch_step, b, moves_dev, flags, nullptr);
     /* Two halves on two streams.  The second half waits for everything queued on the handle's stream so far (the
      * caller's moves, the first half of the previous tick) and, by stream order, for its own previous tick; the first
      * half of the NEXT tick does not wait for it.  So the last, partly filled wave of one kernel runs next to the first
@@ -667,7 +688,7 @@ int pom_batch_step(pom_batch* b, const uint8_t* moves_dev, uint32_t flags)
     for(uint64_t first = 0; first < b->n_envs; first += per, c++)
     {
         const uint64_t count = first + per <= b->n_envs ? per : b->n_envs - first;
-        rc = [&]() -> int { POM_DISPATCH(b, launch_step, b, moves_dev, flags, nullptr, first, count, (c & 1) ? b->s_k2 : b->stream, tile_parts); }();
+        rc = [&]() -> int { POM_DISPATCH_MODE(b, launch_step, b, moves_dev, flags, nullptr, first, count, (c & 1) ? b->s_k2 : b->stream, tile_parts); }();
         if(rc) return rc;
     }
     b->forked = true;
@@ -692,7 +713,7 @@ static int enqueue_step_pipeline(pom_batch* b, const uint8_t* moves_host, uint8_
         CK(cudaMemcpyAsync(reinterpret_cast<uint8_t*>(b->moves_buf) + 4 * first, moves_host + 4 * first, 4 * count, cudaMemcpyHostToDevice, b->s_h2d));
         CK(cudaEventRecord(b->ev_in[c], b->s_h2d));
         CK(cudaStreamWaitEvent(compute, b->ev_in[c], 0));
-        const int rc = [&]() -> int { POM_DISPATCH(b, launch_step, b, reinterpret_cast<const uint8_t*>(b->moves_buf), flags,
+        const int rc = [&]() -> int { POM_DISPATCH_MODE(b, launch_step, b, reinterpret_cast<const uint8_t*>(b->moves_buf), flags,
                                                    status_host ? b->status_buf : nullptr, first, count, compute); }();
         if(rc) return rc;
         if(status_host)
@@ -723,7 +744,7 @@ static int launch_step_zero_copy(pom_batch* b, const uint8_t* moves_host, uint8_
     bool ok = cudaHostGetDevicePointer(&mdev, const_cast<uint8_t*>(moves_host), 0) == cudaSuccess;
     if(ok && status_host) ok = cudaHostGetDevicePointer(&sdev, status_host, 0) == cudaSuccess;
     if(!ok) { cudaGetLastError(); return 1; }
-    return [&]() -> int { POM_DISPATCH(b, launch_step, b, static_cast<const uint8_t*>(mdev), flags, static_cast<uint8_t*>(sdev)); }();
+    return [&]() -> int { POM_DISPATCH_MODE(b, launch_step, b, static_cast<const uint8_t*>(mdev), flags, static_cast<uint8_t*>(sdev)); }();
 }
 
 int pom_batch_step_host_async(pom_batch* b, const uint8_t* moves_host, uint8_t* status_host, uint32_t flags)
@@ -866,14 +887,14 @@ int pom_batch_rollout(pom_batch* b, uint32_t ticks, uint64_t rng_seed, uint32_t 
         uint8_t* mv = reinterpret_cast<uint8_t*>(b->moves_buf);
         for(uint32_t k = 0; k < ticks; k++)
         {
-            rc = [&]() -> int { POM_DISPATCH(b, launch_policy_moves, b, mv, rng_seed, tick0 + k, mask, n_actions, 1u); }();
+            rc = [&]() -> int { POM_DISPATCH_MODE(b, launch_policy_moves, b, mv, rng_seed, tick0 + k, mask, n_actions, 1u); }();
             if(rc) return rc;
-            rc = [&]() -> int { POM_DISPATCH(b, launch_step, b, mv, sflags, nullptr); }();
+            rc = [&]() -> int { POM_DISPATCH_MODE(b, launch_step, b, mv, sflags, nullptr); }();
             if(rc) return rc;
         }
         return POM_OK;
     }
-    POM_DISPATCH(b, launch_rollout, b, ticks, rng_seed, tick0, flags);
+    POM_DISPATCH_MODE(b, launch_rollout, b, ticks, rng_seed, tick0, flags);
 }
 
 int pom_batch_step_seq(pom_batch* b, const uint8_t* moves_dev, uint32_t ticks, uint32_t flags)
@@ -881,7 +902,7 @@ int pom_batch_step_seq(pom_batch* b, const uint8_t* moves_dev, uint32_t ticks, u
     int rc = use(b); if(rc) return rc;
     if(!moves_dev) return fail(POM_E_ARG, "pom_batch_step_seq: null moves");
     if(flags & ~uint32_t(POM_ROLL_NO_RESET | POM_ROLL_CONTINUE_UNDEFINED)) return fail(POM_E_ARG, "pom_batch_step_seq: only POM_ROLL_NO_RESET and POM_ROLL_CONTINUE_UNDEFINED are accepted");
-    POM_DISPATCH(b, launch_rollout, b, ticks, 0, 0, flags, moves_dev);
+    POM_DISPATCH_MODE(b, launch_rollout, b, ticks, 0, 0, flags, moves_dev);
 }
 
 int pom_batch_policy_moves(pom_batch* b, uint8_t* moves_dev, uint64_t seed, uint32_t tick, uint32_t agent_mask)
@@ -890,7 +911,7 @@ int pom_batch_policy_moves(pom_batch* b, uint8_t* moves_dev, uint64_t seed, uint
     if(!moves_dev) return fail(POM_E_ARG, "pom_batch_policy_moves: null moves");
     if(agent_mask == 0 || agent_mask > 0xFu) return fail(POM_E_ARG, "pom_batch_policy_moves: agent_mask must be 1..15");
     rc = ensure_policy(b); if(rc) return rc;
-    POM_DISPATCH(b, launch_policy_moves, b, moves_dev, seed, tick, agent_mask);
+    POM_DISPATCH_MODE(b, launch_policy_moves, b, moves_dev, seed, tick, agent_mask);
 }
 
 int pom_batch_policy_moves_host(pom_batch* b, uint8_t* moves_host, uint64_t seed, uint32_t tick, uint32_t agent_mask)
@@ -914,7 +935,8 @@ int pom_batch_policy_act(pom_batch* b, uint64_t env, int agent, int draw, int* m
     rc = ensure_policy(b); if(rc) return rc;
     DevBuf dev;
     CK(dev.alloc(sizeof(int)));
-    pomk::k_policy_act<<<1, 1, 0, b->stream>>>(b->params(), env, agent, uint32_t(draw), dev.as<int>());
+    if(b->teams) pomk::k_policy_act<true><<<1, 1, 0, b->stream>>>(b->params(), env, agent, uint32_t(draw), dev.as<int>());
+    else pomk::k_policy_act<<<1, 1, 0, b->stream>>>(b->params(), env, agent, uint32_t(draw), dev.as<int>());
     b->launches++;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(move_out, dev.p, sizeof(int), cudaMemcpyDeviceToHost, b->stream));
@@ -969,6 +991,7 @@ int pom_batch_clone(pom_batch* dst, uint64_t first_dst, const pom_batch* src, co
     int rc = use(dst); if(rc) return rc;
     if(!src || !src_idx) return fail(POM_E_ARG, "pom_batch_clone: null argument");
     if(src->device != dst->device) return fail(POM_E_ARG, "pom_batch_clone: handles live on different devices");
+    if(src->teams != dst->teams) return fail(POM_E_ARG, "pom_batch_clone: one handle plays the team game and the other free-for-all (status bytes mean different things)");
     if(src != dst) { rc = use(src); if(rc) return rc; }         /* joins src's second compute stream if a step is in flight there */
     if(first_dst > dst->n_envs || n_dst > dst->n_envs - first_dst) return fail(POM_E_RANGE, "pom_batch_clone: destination range outside the batch");
     for(uint64_t i = 0; i < n_dst; i++) if(src_idx[i] >= src->n_envs) return fail(POM_E_RANGE, "pom_batch_clone: source index outside the batch");
@@ -1000,6 +1023,7 @@ int pom_batch_expand_step(pom_batch* dst, const pom_batch* src, const uint32_t* 
     int rc = use(dst); if(rc) return rc;
     if(!src || !src_idx || src == dst) return fail(POM_E_ARG, "pom_batch_expand_step: bad argument");
     if(src->device != dst->device) return fail(POM_E_ARG, "pom_batch_expand_step: handles live on different devices");
+    if(src->teams != dst->teams) return fail(POM_E_ARG, "pom_batch_expand_step: one handle plays the team game and the other free-for-all (status bytes mean different things)");
     rc = use(src); if(rc) return rc;                              /* joins src's second compute stream if a step is in flight there */
     if(fanout == 0 || fanout > 1296) return fail(POM_E_ARG, "pom_batch_expand_step: fanout must be 1..1296");
     const uint64_t n_children = n_roots * fanout;
@@ -1022,7 +1046,11 @@ int pom_batch_expand_step(pom_batch* dst, const pom_batch* src, const uint32_t* 
      * behind the kernel of a previous expansion that may still be reading the buffer */
     CK(cudaMemcpyAsync(idx_dev, src_idx, n_roots * sizeof(uint32_t), cudaMemcpyHostToDevice, dst->stream));
     CK(cudaStreamSynchronize(src->stream));
-    rc = [&]() -> int { POM_DISPATCH(dst, launch_expand, dst, src, idx_dev, n_children, fanout, flags); }();
+    /* the mode is the source's (the kernel takes no BatchParams); the two handles' modes are equal */
+    rc = [&]() -> int {
+        if(src->teams) return launch_expand<128, true>(dst, src, idx_dev, n_children, fanout, flags);
+        POM_DISPATCH(dst, launch_expand, dst, src, idx_dev, n_children, fanout, flags);
+    }();
     if(rc) return rc;
     /* the call returns with the kernel queued: whatever is queued on the SOURCE handle from now on (a step that rewrites
      * the roots) must wait until the expansion has read them */
@@ -1118,6 +1146,7 @@ int pom_batch_generate_moves(pom_batch* b, uint8_t* moves_dev, uint64_t seed, ui
 }
 
 uint64_t pom_batch_size(const pom_batch* b) { return b ? b->n_envs : 0; }
+int      pom_batch_teams(const pom_batch* b) { return b ? (b->teams ? 1 : 0) : fail(POM_E_ARG, "pom_batch_teams: null handle"); }
 int      pom_batch_device(const pom_batch* b) { return b ? b->device : -1; }
 void*    pom_batch_stream(const pom_batch* b) { return b ? (void*)b->stream : nullptr; }
 void*    pom_batch_stats_device_ptr(const pom_batch* b) { return b ? (void*)b->stats : nullptr; }

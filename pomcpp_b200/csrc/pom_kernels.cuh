@@ -332,7 +332,9 @@ __device__ __forceinline__ void warp_explode_due(uint8_t* sslice, uint8_t* rec, 
     }
 }
 
-/* bboard::Step (+ Environment::Step's bookkeeping unless raw) for the env of every lane with `step` set */
+/* bboard::Step (+ Environment::Step's bookkeeping unless raw; TEAMS: the team game's, pomcore::env_post) for the env of
+ * every lane with `step` set */
+template<bool TEAMS = false>
 __device__ __forceinline__ void warp_tick(uint8_t* sslice, uint8_t* rec, uint32_t m, bool step, bool raw, uint8_t* wlist,
                                           int invalid_mask = pomcore::F_INVALID_MASK)
 {
@@ -345,7 +347,7 @@ __device__ __forceinline__ void warp_tick(uint8_t* sslice, uint8_t* rec, uint32_
     if(step)
     {
         if(flags & invalid_mask) rec[R_STATUS] |= POM_STATUS_INVALID;
-        if(!raw) pomcore::env_post(rec);
+        if(!raw) pomcore::env_post<TEAMS>(rec);
     }
 }
 
@@ -405,7 +407,9 @@ template<int TPB> struct TileScratch {
 };
 
 /* ---------------------------------------------------------------- K1: per-tick kernel */
-template<int TPB>
+/* TEAMS (here and in every kernel below that takes it): the 2v2 team game - its episode rule (pomcore::env_post) and its
+ * SimpleAgent (pompolicy::plan_agent).  The mode belongs to the handle; the free-for-all images are the default. */
+template<int TPB, bool TEAMS = false>
 __global__ void __launch_bounds__(TPB) k_step(BatchParams P, const uint32_t* __restrict__ moves, uint32_t flags, uint8_t* __restrict__ status_out)
 {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -436,8 +440,8 @@ __global__ void __launch_bounds__(TPB) k_step(BatchParams P, const uint32_t* __r
     uint8_t* rec = sslice + lane * POM_REC_BYTES;
     /* finished envs are skipped (environment.cpp:125) unless raw; invalid envs always freeze */
     const bool stepped = active && !(rec[R_STATUS] & (raw ? POM_STATUS_INVALID : (POM_STATUS_DONE | POM_STATUS_INVALID)));
-    warp_tick(sslice, rec, m, stepped, raw, smem + TileScratch<TPB>::OFF_LIST + 8u * warp,
-              (flags & POM_STEP_CONTINUE_UNDEFINED) ? pomcore::F_INVALID_MASK_CONTINUE : pomcore::F_INVALID_MASK);
+    warp_tick<TEAMS>(sslice, rec, m, stepped, raw, smem + TileScratch<TPB>::OFF_LIST + 8u * warp,
+                     (flags & POM_STEP_CONTINUE_UNDEFINED) ? pomcore::F_INVALID_MASK_CONTINUE : pomcore::F_INVALID_MASK);
     EpisodeAcc acc;
     acc.steps = stepped ? 1u : 0u;
     uint32_t st_end = active ? rec[R_STATUS] : 0u;
@@ -527,7 +531,7 @@ template<int NBUF> struct RingScratch {
  * the two-stream overlap).  The same treatment of the compact-I/O configuration was measured 6-15 % SLOWER than the
  * generic image in three variants (all of io constant; the flags only; joint + bulk only) and is not built: what the
  * compiler makes of this loop body is not monotone in what it knows (see also FREEZE below). */
-template<int NW, int NBUF, bool OBS, bool FREEZE, bool SPEC = false>
+template<int NW, int NBUF, bool OBS, bool FREEZE, bool SPEC = false, bool TEAMS = false>
 __global__ void __launch_bounds__((NW + 1) * 32, 1) k_step_ws(BatchParams P, StepIO io_in, uint32_t flags_in)
 {
     const uint32_t flags = SPEC ? uint32_t(POM_STEP_AUTORESET | POM_STEP_COUNT) : flags_in;
@@ -627,8 +631,8 @@ __global__ void __launch_bounds__((NW + 1) * 32, 1) k_step_ws(BatchParams P, Ste
          * compile-time constant per branch of `raw`.  tools/ab keeps the builds of that A/B.) */
         const bool stepped = active && !(rec[R_STATUS] & ((raw ? POM_STATUS_INVALID : (POM_STATUS_DONE | POM_STATUS_INVALID)) |
                                                           (FREEZE ? POM_STATUS_TRUNCATED : 0)));
-        warp_tick(sslice, rec, m, stepped, raw, sslice + R::SLICE_BYTES + 128u,
-                  (flags & POM_STEP_CONTINUE_UNDEFINED) ? pomcore::F_INVALID_MASK_CONTINUE : pomcore::F_INVALID_MASK);
+        warp_tick<TEAMS>(sslice, rec, m, stepped, raw, sslice + R::SLICE_BYTES + 128u,
+                         (flags & POM_STEP_CONTINUE_UNDEFINED) ? pomcore::F_INVALID_MASK_CONTINUE : pomcore::F_INVALID_MASK);
         acc.steps += stepped ? 1u : 0u;
         uint32_t st_end = active ? rec[R_STATUS] : 0u;
         if(flags & POM_STEP_AUTORESET)
@@ -776,7 +780,7 @@ struct GlobalAgentStore {
 
 /* per-tick mode: moves[env] byte a <- SimpleAgent::act for every agent a in `mask` of every running env (IDLE for a dead
  * agent); the other bytes are kept.  Records are staged read-only with the same per-warp bulk load as k_step. */
-template<int TPB>
+template<int TPB, bool TEAMS = false>
 __global__ void __launch_bounds__(TPB) k_policy_moves(BatchParams P, uint32_t* __restrict__ moves, uint64_t seed, uint32_t tick, uint32_t mask,
                                                      uint32_t gen_actions, uint32_t freeze_truncated)
 {
@@ -807,7 +811,7 @@ __global__ void __launch_bounds__(TPB) k_policy_moves(BatchParams P, uint32_t* _
     {
         GlobalAgentStore S{ P.policy + env, P.policy_stride };
         S.claim(ep);
-        m = pompolicy::simple_moves(rec, mask, m, draws, S);
+        m = pompolicy::simple_moves<TEAMS>(rec, mask, m, draws, S);
         moves[env] = m;
     }
     else if(active && gen_actions) moves[env] = m;
@@ -818,7 +822,7 @@ __global__ void __launch_bounds__(TPB) k_policy_moves(BatchParams P, uint32_t* _
  * POLICY = true : the agents in `policy_mask` play SimpleAgent, the others stay uniform random. */
 /* SPEC: the image of the headline rollout (uniform{0..5} agents from the counter RNG, auto-reset, default handling of
  * the undefined states) with those choices known at compile time */
-template<int TPB, bool POLICY, bool SPEC = false>
+template<int TPB, bool POLICY, bool SPEC = false, bool TEAMS = false>
 __global__ void __launch_bounds__(TPB) k_rollout(BatchParams P, uint32_t ticks, uint64_t seed, uint32_t tick0,
                                                 uint32_t n_actions_in, uint32_t roll_flags_in, uint32_t policy_mask,
                                                 const uint32_t* __restrict__ move_seq_in)
@@ -877,11 +881,11 @@ __global__ void __launch_bounds__(TPB) k_rollout(BatchParams P, uint32_t ticks, 
 #pragma unroll
                 for(int a = 0; a < 4; a++)
                     draws |= (((uint32_t(h >> (16 * a)) & 0xFFFFu) * 5u) >> 16) << (8 * a);
-                m = pompolicy::simple_moves(rec, policy_mask, m, draws, agents);
+                m = pompolicy::simple_moves<TEAMS>(rec, policy_mask, m, draws, agents);
             }
             acc.steps++;
         }
-        warp_tick(sslice, rec, m, stepped, false, smem + TileScratch<TPB>::OFF_LIST + 8u * warp, invalid_mask);
+        warp_tick<TEAMS>(sslice, rec, m, stepped, false, smem + TileScratch<TPB>::OFF_LIST + 8u * warp, invalid_mask);
         const uint32_t st = finish_and_reset(sslice, rec, P, env, active && stepped, !no_reset, ep_now, acc);
         /* a new episode starts with four new agents */
         if(POLICY && stepped && !no_reset && (st & (POM_STATUS_DONE | POM_STATUS_TRUNCATED | POM_STATUS_INVALID))) agents.clear(ep_now);
@@ -898,6 +902,7 @@ __global__ void __launch_bounds__(TPB) k_rollout(BatchParams P, uint32_t ticks, 
 }
 
 /* SimpleAgent::act for ONE agent of ONE env with a caller-chosen draw (the host mirror's agents::SimpleAgent) */
+template<bool TEAMS = false>
 __global__ void k_policy_act(BatchParams P, uint64_t env, int agent, uint32_t draw, int* move_out)
 {
     const uint8_t* rec = P.recs + env * POM_REC_BYTES;
@@ -905,7 +910,7 @@ __global__ void k_policy_act(BatchParams P, uint64_t env, int agent, uint32_t dr
     S.claim(P.episodes[env]);
     const pompolicy::Boards B = pompolicy::make_boards(rec);
     pompolicy::SimpleSt st = S.load(agent);
-    *move_out = int(pompolicy::simple_act(rec, B, agent, st, draw));
+    *move_out = int(pompolicy::simple_act<TEAMS>(rec, B, agent, st, draw));
     S.store(agent, st);
 }
 
@@ -972,7 +977,7 @@ __global__ void k_fill_from_templates(BatchParams P)
  * replicate them from registers into the 32 records - 96 conflict-free shared-memory stores per lane, no load between
  * them.  (The first form had every lane copy its own record word by word: 73 dependent load -> store pairs per lane,
  * one in flight at a time, 0.55 of the HBM write peak.) */
-template<int TPB>
+template<int TPB, bool TEAMS = false>
 __global__ void __launch_bounds__(TPB) k_expand_step(uint8_t* __restrict__ dst, const uint8_t* __restrict__ src,
                                                     const uint32_t* __restrict__ src_idx, uint64_t n_children,
                                                     uint32_t fanout, uint32_t flags)
@@ -1024,8 +1029,8 @@ __global__ void __launch_bounds__(TPB) k_expand_step(uint8_t* __restrict__ dst, 
         m = moves_of_joint(j);
         stepped = !(rec[R_STATUS] & (raw ? POM_STATUS_INVALID : (POM_STATUS_DONE | POM_STATUS_INVALID)));
     }
-    warp_tick(sslice, rec, m, stepped, raw, smem + TileScratch<TPB>::OFF_LIST + 8u * warp,
-              (flags & POM_STEP_CONTINUE_UNDEFINED) ? pomcore::F_INVALID_MASK_CONTINUE : pomcore::F_INVALID_MASK);
+    warp_tick<TEAMS>(sslice, rec, m, stepped, raw, smem + TileScratch<TPB>::OFF_LIST + 8u * warp,
+                     (flags & POM_STEP_CONTINUE_UNDEFINED) ? pomcore::F_INVALID_MASK_CONTINUE : pomcore::F_INVALID_MASK);
     if(n_here == 32u)
     {
         fence_proxy_async();

@@ -292,7 +292,10 @@ struct Plan {
     bb_t     region;        /* FLEE: the cells MoveTowardsSafePlace scans                                        */
 };
 
-/* phase 1: which branch of _Decide is agent `id` in */
+/* phase 1: which branch of _Decide is agent `id` in.
+ * TEAMS: the team game (env_post): the teammate id ^ 2 is no enemy - neither for IsAdjacentEnemy nor as the target of
+ * MoveTowardsEnemy; everything else is the same agent */
+template<bool TEAMS = false>
 POM_HD Plan plan_agent(const uint8_t* r, int id, const SimpleSt& st, uint32_t draw)
 {
     Plan pl;
@@ -311,7 +314,7 @@ POM_HD Plan plan_agent(const uint8_t* r, int id, const SimpleSt& st, uint32_t dr
         int dmin = 99, target = -1;
         for(int i = 0; i < 4; i++)
         {
-            if(i == id || (r[R_AFLAGS + i] & AF_DEAD)) continue;
+            if(i == id || (TEAMS && i == (id ^ 2)) || (r[R_AFLAGS + i] & AF_DEAD)) continue;
             const int dx = int(r[R_APOS + i] & 15u) - x, dy = int(r[R_APOS + i] >> 4) - y;
             const int d = (dx < 0 ? -dx : dx) + (dy < 0 ? -dy : dy);
             if(d < dmin) dmin = d;
@@ -465,11 +468,12 @@ POM_HD void remember_position(const uint8_t* r, int id, SimpleSt& st, uint32_t m
 }
 
 /* SimpleAgent::act for ONE agent */
+template<bool TEAMS = false>
 POM_HD uint32_t simple_act(const uint8_t* r, const Boards& B, int id, SimpleSt& st, uint32_t draw)
 {
     Plan pl[4];
     for(int a = 0; a < 4; a++) pl[a].kind = K_NONE;
-    pl[id] = plan_agent(r, id, st, draw);
+    pl[id] = plan_agent<TEAMS>(r, id, st, draw);
     run_floods(r, B, pl, (pl[id].kind == K_FLEE || pl[id].target != 0xFFu) ? 1u << id : 0u);
     const uint32_t m = finish_agent(r, id, pl[id], st, draw);
     remember_position(r, id, st, m);
@@ -480,7 +484,7 @@ POM_HD uint32_t simple_act(const uint8_t* r, const Boards& B, int id, SimpleSt& 
  * bytes of the masked agents replaced (IDLE for a dead agent, whose slot the reference leaves unwritten).
  * `draws` = pom_rng_moves(seed, env, tick, 5): byte a is agent a's uniform{0..4} draw.  `S` gives access to the
  * four agent states: S.load(a) / S.store(a, st) (an array on the host, shared or global memory in the kernels). */
-template<class Store>
+template<bool TEAMS = false, class Store>
 POM_HD uint32_t simple_moves(const uint8_t* r, uint32_t mask, uint32_t moves, uint32_t draws, Store& S)
 {
     const Boards B = make_boards(r);
@@ -492,7 +496,7 @@ POM_HD uint32_t simple_moves(const uint8_t* r, uint32_t mask, uint32_t moves, ui
         pl[a].kind = K_NONE;
         if(((mask >> a) & 1u) && !(r[R_AFLAGS + a] & AF_DEAD))
         {
-            pl[a] = plan_agent(r, a, S.load(a), byte_of(draws, a));
+            pl[a] = plan_agent<TEAMS>(r, a, S.load(a), byte_of(draws, a));
             if(pl[a].kind == K_FLEE || pl[a].target != 0xFFu) jobs |= 1u << a;
         }
     }

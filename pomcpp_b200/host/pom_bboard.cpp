@@ -306,8 +306,9 @@ int Environment::GetWinner() { return agentWon; }
 Move Environment::GetLastMove(int agentID) { return lastMoves[agentID]; }
 
 /* ---- BatchEnvironment ---- */
-BatchEnvironment::BatchEnvironment(size_t nGames, int device, uint64_t envOffset, uint32_t nTemplates, int firstSeed, uint32_t maxTicks)
-    : n(nGames)
+BatchEnvironment::BatchEnvironment(size_t nGames, int device, uint64_t envOffset, uint32_t nTemplates, int firstSeed, uint32_t maxTicks,
+                                   bool teams)
+    : n(nGames), teams(teams)
 {
     pom_init_desc d;
     std::memset(&d, 0, sizeof(d));
@@ -315,6 +316,7 @@ BatchEnvironment::BatchEnvironment(size_t nGames, int device, uint64_t envOffset
     d.n_templates = nTemplates;
     d.first_seed = firstSeed;
     d.max_ticks = maxTicks;
+    d.flags = teams ? POM_INIT_TEAMS : 0;
     check(pom_batch_init(&handle, device, n, &d), "pom_batch_init");
     movebuf.resize(4 * n);
 }
@@ -425,7 +427,13 @@ bool BatchEnvironment::IsDraw(size_t i) { Refresh(); return (status[i] & POM_STA
 int BatchEnvironment::GetWinner(size_t i)
 {
     Refresh();
-    if(!(status[i] & POM_STATUS_DONE) || (status[i] & POM_STATUS_DRAW)) return -1;
+    if(teams || !(status[i] & POM_STATUS_DONE) || (status[i] & POM_STATUS_DRAW)) return -1;
+    return (status[i] & POM_STATUS_WINNER_MASK) >> POM_STATUS_WINNER_SHIFT;
+}
+int BatchEnvironment::GetWinningTeam(size_t i)
+{
+    Refresh();
+    if(!teams || !(status[i] & POM_STATUS_DONE) || (status[i] & POM_STATUS_DRAW)) return -1;
     return (status[i] & POM_STATUS_WINNER_MASK) >> POM_STATUS_WINNER_SHIFT;
 }
 
