@@ -237,6 +237,23 @@ int  pom_batch_policy_reset(pom_batch* b);                          /* all agent
 int  pom_batch_policy_download(pom_batch* b, uint64_t first, uint64_t count, pom_simple_agent* out);
 int  pom_batch_policy_upload(pom_batch* b, uint64_t first, uint64_t count, const pom_simple_agent* in);
 
+/* Fog of war for the device SimpleAgent.  With a policy view v >= 0 every act of agent a is
+ *     SimpleAgent::act( N_a( fog_state(state, a, v) ) )
+ * where fog_state is the fogged State of pom_batch_observe (the unclamped square window [x - v, x + v] x [y - v, y + v]
+ * around the agent's stored position: cells outside it become FOG, bombs outside it or off the board are dropped, other
+ * agents outside it or dead are hidden with x = y = -1), and N_a makes every hidden agent absent: dead, at (0, 0) (as
+ * SimpleActOnDevice does for the host agents of BatchEnvironment::SetViewRange).  The agent is otherwise the same one,
+ * quirks included, team-aware on a team handle; its draw and its memory are those of the full-state agent.  It never reads
+ * the flame queue.  So an enemy outside the window is not hunted or bombed and a bomb outside it does not make the agent
+ * flee; with v = 0 the agent sees only its own cell.
+ * The view is a property of the handle that may change between calls; it applies to every call made after it that runs
+ * the device SimpleAgent: pom_batch_policy_moves[_host], pom_batch_rollout with POM_ROLL_SIMPLE (the fused and the
+ * tick-by-tick path), pom_batch_policy_act.  A negative view (the default, -1) means the full state: the agent of the calls
+ * above.  Any view >= 0 is accepted; from 15 on the window holds every position.  pom_batch_clone and
+ * pom_batch_expand_step do not look at it.  The getter writes the view last set to *view_out. */
+int  pom_batch_set_policy_view(pom_batch* b, int view);
+int  pom_batch_get_policy_view(const pom_batch* b, int* view_out);
+
 /* state copy for tree search (the reference copies the POD State by assignment, README.md:4):
  * dst env first_dst + i <- src env src_idx[i] (HOST array of n_dst indices).  dst may equal src.    */
 int  pom_batch_clone(pom_batch* dst, uint64_t first_dst, const pom_batch* src, const uint32_t* src_idx, uint64_t n_dst);

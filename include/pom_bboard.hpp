@@ -267,6 +267,10 @@ public:
      * exposed (the "potentially fogged board state" of bboard.hpp:529, which the reference never implements);
      * view < 0 (default) = full observability, as in the reference */
     void SetViewRange(int view) { viewRange = view; }
+    /* fog of war for the device SimpleAgent of Step(moves, simpleMask, seed) and Rollout(..., simpleMask): with view >= 0
+     * it plays on what it sees through its window of `view` cells (pom_batch_set_policy_view); view < 0 (default) = the
+     * full state.  Independent of SetViewRange, which applies to the host agents of Step(agents) only */
+    void SetSimpleViewRange(int view);
     /* the State of every game as agent `agentID` observes it */
     std::vector<State> Observe(int agentID, int view);
     /* host copies */

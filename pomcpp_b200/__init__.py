@@ -133,6 +133,8 @@ def lib():
         L.pom_batch_generate_moves.argtypes = [vp, vp, u64, u32, u32]
         L.pom_batch_size.restype = u64
         L.pom_batch_teams.argtypes = [vp]
+        L.pom_batch_set_policy_view.argtypes = [vp, i32]
+        L.pom_batch_get_policy_view.argtypes = [vp, C.POINTER(C.c_int)]
         L.pom_batch_size.argtypes = [vp]
         L.pom_batch_device.argtypes = [vp]
         for f in ("pom_batch_stream", "pom_batch_stats_device_ptr", "pom_batch_records_device_ptr"):
@@ -211,6 +213,18 @@ class Batch:
         r = lib().pom_batch_teams(self.h)
         _ck(min(r, 0))
         return r == 1
+
+    def set_policy_view(self, view):
+        """fog of war for the device SimpleAgent (pom_batch_set_policy_view): with view >= 0 every later call that runs it
+        (policy_moves[_host], rollout with ROLL_SIMPLE, policy_act) plays it on what each agent sees through its square
+        window of `view` cells; view < 0 (the default, -1) = the full state"""
+        _ck(lib().pom_batch_set_policy_view(self.h, int(view)))
+
+    def policy_view(self):
+        """the view last set by set_policy_view (-1 if never set)"""
+        v = C.c_int(0)
+        _ck(lib().pom_batch_get_policy_view(self.h, C.byref(v)))
+        return v.value
     def reset(self): _ck(lib().pom_batch_reset(self.h))
 
     def upload(self, states, status=None, first=0):

@@ -70,6 +70,8 @@ struct pom_batch {
     int       step_kernel = 0;                 /* 0 = k_step_ws (persistent, warp-specialised), 1 = k_step (one CTA per tile); POM_STEP_KERNEL=tile */
     bool      teams = false;                   /* POM_INIT_TEAMS: the 2v2 team game, fixed for the handle's life; every stepping or
                                                   acting launch takes the kernel images of this mode (POM_DISPATCH_MODE) */
+    int       policy_view = -1;                /* pom_batch_set_policy_view: >= 0 = the device SimpleAgent plays under fog of war
+                                                  with this view (the FOG images, POM_DISPATCH_POLICY), < 0 = on the full state */
     uint8_t*  recs = nullptr;
     uint8_t*  templates = nullptr;
     uint32_t* episodes = nullptr;
@@ -132,8 +134,14 @@ int use(const pom_batch* cb, bool join = true)
 /* The dynamic shared-memory limit of a kernel is a per-device attribute: remember it per handle (one handle = one
  * device), not in a process-wide flag, so that handles on other GPUs and other host threads set it for themselves. */
 enum { ATTR_STEP = 1, ATTR_ROLLOUT = 2, ATTR_ROLLOUT_POLICY = 4, ATTR_POLICY_MOVES = 8, ATTR_EXPAND = 16, ATTR_OBS = 32, ATTR_ROLLOUT_SPEC = 64, ATTR_OBS_CROPPED = 128 };
-/* the bit of a kernel's team image */
-constexpr uint32_t attr_bit(uint32_t which, bool teams) { return teams ? which << 8 : which; }
+/* the bit of a kernel's team image, and of its FOG image (bits 16..23 for free-for-all, 24..31 for the team game) */
+constexpr uint32_t attr_bit(uint32_t which, bool teams, bool fog = false) { return (fog ? which << 16 : which) << (teams ? 8 : 0); }
+
+/* the handle's policy view as the FOG images take it: in the spare bits of the agent mask or draw (pomk::POLICY_VIEW_SHIFT) */
+uint32_t policy_view_bits(const pom_batch* b)
+{
+    return uint32_t(b->policy_view > 15 ? 15 : b->policy_view) << pomk::POLICY_VIEW_SHIFT;
+}
 
 template<typename K>
 int set_smem(pom_batch* b, uint32_t which, K kernel, uint32_t bytes)
@@ -315,7 +323,7 @@ int launch_step(pom_batch* b, const uint8_t* moves_dev, uint32_t flags, uint8_t*
     return POM_OK;
 }
 
-template<int TPB, bool TEAMS = false>
+template<int TPB, bool TEAMS = false, bool FOG = false>
 int launch_rollout(pom_batch* b, uint32_t ticks, uint64_t seed, uint32_t tick0, uint32_t flags, const uint8_t* move_seq = nullptr)
 {
     const uint32_t n_actions = (flags & POM_ROLL_HARMLESS) ? 5u : 6u, no_reset = flags & (POM_ROLL_NO_RESET | POM_ROLL_CONTINUE_UNDEFINED);
@@ -323,9 +331,10 @@ int launch_rollout(pom_batch* b, uint32_t ticks, uint64_t seed, uint32_t tick0, 
     const unsigned grid = unsigned((b->n_envs + TPB - 1) / TPB);
     if(mask)
     {
-        int rc = set_smem(b, attr_bit(ATTR_ROLLOUT_POLICY, TEAMS), pomk::k_rollout<TPB, true, false, TEAMS>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
+        int rc = set_smem(b, attr_bit(ATTR_ROLLOUT_POLICY, TEAMS, FOG), pomk::k_rollout<TPB, true, false, TEAMS, FOG>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
         rc = ensure_policy(b); if(rc) return rc;
-        pomk::k_rollout<TPB, true, false, TEAMS><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), ticks, seed, tick0, n_actions, no_reset, mask, nullptr);
+        pomk::k_rollout<TPB, true, false, TEAMS, FOG><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), ticks, seed, tick0, n_actions, no_reset,
+                                                                                                     FOG ? mask | policy_view_bits(b) : mask, nullptr);
     }
     else if(!TEAMS && n_actions == 6u && no_reset == 0u && !move_seq && !b->no_spec)      /* the SPEC image is free-for-all only */
     {
@@ -342,12 +351,13 @@ int launch_rollout(pom_batch* b, uint32_t ticks, uint64_t seed, uint32_t tick0, 
     return POM_OK;
 }
 
-template<int TPB, bool TEAMS = false>
+template<int TPB, bool TEAMS = false, bool FOG = false>
 int launch_policy_moves(pom_batch* b, uint8_t* moves_dev, uint64_t seed, uint32_t tick, uint32_t mask, uint32_t gen_actions = 0, uint32_t freeze_truncated = 0)
 {
-    { int rc = set_smem(b, attr_bit(ATTR_POLICY_MOVES, TEAMS), pomk::k_policy_moves<TPB, TEAMS>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc; }
+    { int rc = set_smem(b, attr_bit(ATTR_POLICY_MOVES, TEAMS, FOG), pomk::k_policy_moves<TPB, TEAMS, FOG>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc; }
     const unsigned grid = unsigned((b->n_envs + TPB - 1) / TPB);
-    pomk::k_policy_moves<TPB, TEAMS><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), reinterpret_cast<uint32_t*>(moves_dev), seed, tick, mask, gen_actions, freeze_truncated);
+    pomk::k_policy_moves<TPB, TEAMS, FOG><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), reinterpret_cast<uint32_t*>(moves_dev), seed, tick,
+                                                                                            FOG ? mask | policy_view_bits(b) : mask, gen_actions, freeze_truncated);
     b->launches++;
     CK(cudaGetLastError());
     return POM_OK;
@@ -446,6 +456,17 @@ bool local_cpus(int device, cpu_set_t* set)
     do { \
         if((h)->teams) return fn<128, true>(__VA_ARGS__); \
         POM_DISPATCH(h, fn, __VA_ARGS__); \
+    } while(0)
+/* the same for the launches that run the device SimpleAgent: a handle with a policy view takes the FOG images of its mode,
+ * which also exist for the default geometry only */
+#define POM_DISPATCH_POLICY(h, fn, ...) \
+    do { \
+        if((h)->policy_view >= 0) \
+        { \
+            if((h)->teams) return fn<128, true, true>(__VA_ARGS__); \
+            return fn<128, false, true>(__VA_ARGS__); \
+        } \
+        POM_DISPATCH_MODE(h, fn, __VA_ARGS__); \
     } while(0)
 
 extern "C" {
@@ -887,13 +908,14 @@ int pom_batch_rollout(pom_batch* b, uint32_t ticks, uint64_t rng_seed, uint32_t 
         uint8_t* mv = reinterpret_cast<uint8_t*>(b->moves_buf);
         for(uint32_t k = 0; k < ticks; k++)
         {
-            rc = [&]() -> int { POM_DISPATCH_MODE(b, launch_policy_moves, b, mv, rng_seed, tick0 + k, mask, n_actions, 1u); }();
+            rc = [&]() -> int { POM_DISPATCH_POLICY(b, launch_policy_moves, b, mv, rng_seed, tick0 + k, mask, n_actions, 1u); }();
             if(rc) return rc;
             rc = [&]() -> int { POM_DISPATCH_MODE(b, launch_step, b, mv, sflags, nullptr); }();
             if(rc) return rc;
         }
         return POM_OK;
     }
+    if(mask) POM_DISPATCH_POLICY(b, launch_rollout, b, ticks, rng_seed, tick0, flags);
     POM_DISPATCH_MODE(b, launch_rollout, b, ticks, rng_seed, tick0, flags);
 }
 
@@ -911,7 +933,7 @@ int pom_batch_policy_moves(pom_batch* b, uint8_t* moves_dev, uint64_t seed, uint
     if(!moves_dev) return fail(POM_E_ARG, "pom_batch_policy_moves: null moves");
     if(agent_mask == 0 || agent_mask > 0xFu) return fail(POM_E_ARG, "pom_batch_policy_moves: agent_mask must be 1..15");
     rc = ensure_policy(b); if(rc) return rc;
-    POM_DISPATCH_MODE(b, launch_policy_moves, b, moves_dev, seed, tick, agent_mask);
+    POM_DISPATCH_POLICY(b, launch_policy_moves, b, moves_dev, seed, tick, agent_mask);
 }
 
 int pom_batch_policy_moves_host(pom_batch* b, uint8_t* moves_host, uint64_t seed, uint32_t tick, uint32_t agent_mask)
@@ -935,7 +957,13 @@ int pom_batch_policy_act(pom_batch* b, uint64_t env, int agent, int draw, int* m
     rc = ensure_policy(b); if(rc) return rc;
     DevBuf dev;
     CK(dev.alloc(sizeof(int)));
-    if(b->teams) pomk::k_policy_act<true><<<1, 1, 0, b->stream>>>(b->params(), env, agent, uint32_t(draw), dev.as<int>());
+    if(b->policy_view >= 0)
+    {
+        const uint32_t arg = uint32_t(draw) | policy_view_bits(b);
+        if(b->teams) pomk::k_policy_act<true, true><<<1, 1, 0, b->stream>>>(b->params(), env, agent, arg, dev.as<int>());
+        else pomk::k_policy_act<false, true><<<1, 1, 0, b->stream>>>(b->params(), env, agent, arg, dev.as<int>());
+    }
+    else if(b->teams) pomk::k_policy_act<true><<<1, 1, 0, b->stream>>>(b->params(), env, agent, uint32_t(draw), dev.as<int>());
     else pomk::k_policy_act<<<1, 1, 0, b->stream>>>(b->params(), env, agent, uint32_t(draw), dev.as<int>());
     b->launches++;
     CK(cudaGetLastError());
@@ -1147,6 +1175,20 @@ int pom_batch_generate_moves(pom_batch* b, uint8_t* moves_dev, uint64_t seed, ui
 
 uint64_t pom_batch_size(const pom_batch* b) { return b ? b->n_envs : 0; }
 int      pom_batch_teams(const pom_batch* b) { return b ? (b->teams ? 1 : 0) : fail(POM_E_ARG, "pom_batch_teams: null handle"); }
+
+int pom_batch_set_policy_view(pom_batch* b, int view)
+{
+    if(!b) return fail(POM_E_ARG, "pom_batch_set_policy_view: null handle");
+    b->policy_view = view;
+    return POM_OK;
+}
+
+int pom_batch_get_policy_view(const pom_batch* b, int* view_out)
+{
+    if(!b || !view_out) return fail(POM_E_ARG, "pom_batch_get_policy_view: null argument");
+    *view_out = b->policy_view;
+    return POM_OK;
+}
 int      pom_batch_device(const pom_batch* b) { return b ? b->device : -1; }
 void*    pom_batch_stream(const pom_batch* b) { return b ? (void*)b->stream : nullptr; }
 void*    pom_batch_stats_device_ptr(const pom_batch* b) { return b ? (void*)b->stats : nullptr; }

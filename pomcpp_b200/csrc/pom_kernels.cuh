@@ -778,9 +778,15 @@ struct GlobalAgentStore {
     }
 };
 
+/* FOG (k_policy_moves, k_rollout with POLICY, k_policy_act): the SimpleAgents play under fog of war
+ * (pom_batch_set_policy_view, pompolicy::simple_moves).  The view, 0..15, is a run-time value that travels in spare bits
+ * of an existing argument: bits POLICY_VIEW_SHIFT.. of the agent mask, of k_policy_act's draw.  (A view of 15 sees every
+ * position a record can hold, so larger views are passed as 15.) */
+constexpr uint32_t POLICY_VIEW_SHIFT = 8;
+
 /* per-tick mode: moves[env] byte a <- SimpleAgent::act for every agent a in `mask` of every running env (IDLE for a dead
  * agent); the other bytes are kept.  Records are staged read-only with the same per-warp bulk load as k_step. */
-template<int TPB, bool TEAMS = false>
+template<int TPB, bool TEAMS = false, bool FOG = false>
 __global__ void __launch_bounds__(TPB) k_policy_moves(BatchParams P, uint32_t* __restrict__ moves, uint64_t seed, uint32_t tick, uint32_t mask,
                                                      uint32_t gen_actions, uint32_t freeze_truncated)
 {
@@ -811,7 +817,8 @@ __global__ void __launch_bounds__(TPB) k_policy_moves(BatchParams P, uint32_t* _
     {
         GlobalAgentStore S{ P.policy + env, P.policy_stride };
         S.claim(ep);
-        m = pompolicy::simple_moves<TEAMS>(rec, mask, m, draws, S);
+        if constexpr(FOG) m = pompolicy::simple_moves<TEAMS, true>(rec, mask, m, draws, S, int(mask >> POLICY_VIEW_SHIFT));
+        else m = pompolicy::simple_moves<TEAMS>(rec, mask, m, draws, S);
         moves[env] = m;
     }
     else if(active && gen_actions) moves[env] = m;
@@ -822,7 +829,7 @@ __global__ void __launch_bounds__(TPB) k_policy_moves(BatchParams P, uint32_t* _
  * POLICY = true : the agents in `policy_mask` play SimpleAgent, the others stay uniform random. */
 /* SPEC: the image of the headline rollout (uniform{0..5} agents from the counter RNG, auto-reset, default handling of
  * the undefined states) with those choices known at compile time */
-template<int TPB, bool POLICY, bool SPEC = false, bool TEAMS = false>
+template<int TPB, bool POLICY, bool SPEC = false, bool TEAMS = false, bool FOG = false>
 __global__ void __launch_bounds__(TPB) k_rollout(BatchParams P, uint32_t ticks, uint64_t seed, uint32_t tick0,
                                                 uint32_t n_actions_in, uint32_t roll_flags_in, uint32_t policy_mask,
                                                 const uint32_t* __restrict__ move_seq_in)
@@ -881,7 +888,8 @@ __global__ void __launch_bounds__(TPB) k_rollout(BatchParams P, uint32_t ticks, 
 #pragma unroll
                 for(int a = 0; a < 4; a++)
                     draws |= (((uint32_t(h >> (16 * a)) & 0xFFFFu) * 5u) >> 16) << (8 * a);
-                m = pompolicy::simple_moves<TEAMS>(rec, policy_mask, m, draws, agents);
+                if constexpr(FOG) m = pompolicy::simple_moves<TEAMS, true>(rec, policy_mask, m, draws, agents, int(policy_mask >> POLICY_VIEW_SHIFT));
+                else m = pompolicy::simple_moves<TEAMS>(rec, policy_mask, m, draws, agents);
             }
             acc.steps++;
         }
@@ -902,7 +910,7 @@ __global__ void __launch_bounds__(TPB) k_rollout(BatchParams P, uint32_t ticks, 
 }
 
 /* SimpleAgent::act for ONE agent of ONE env with a caller-chosen draw (the host mirror's agents::SimpleAgent) */
-template<bool TEAMS = false>
+template<bool TEAMS = false, bool FOG = false>
 __global__ void k_policy_act(BatchParams P, uint64_t env, int agent, uint32_t draw, int* move_out)
 {
     const uint8_t* rec = P.recs + env * POM_REC_BYTES;
@@ -910,7 +918,8 @@ __global__ void k_policy_act(BatchParams P, uint64_t env, int agent, uint32_t dr
     S.claim(P.episodes[env]);
     const pompolicy::Boards B = pompolicy::make_boards(rec);
     pompolicy::SimpleSt st = S.load(agent);
-    *move_out = int(pompolicy::simple_act<TEAMS>(rec, B, agent, st, draw));
+    if constexpr(FOG) *move_out = int(pompolicy::simple_act<TEAMS, true>(rec, B, agent, st, draw & 0xFFu, int(draw >> POLICY_VIEW_SHIFT)));
+    else *move_out = int(pompolicy::simple_act<TEAMS>(rec, B, agent, st, draw));
     S.store(agent, st);
 }
 

@@ -410,6 +410,11 @@ size_t BatchEnvironment::StepSequence(const Move* moves, uint32_t ticks)
     return running;
 }
 
+void BatchEnvironment::SetSimpleViewRange(int view)
+{
+    check(pom_batch_set_policy_view(handle, view), "pom_batch_set_policy_view");
+}
+
 pom_stats BatchEnvironment::Rollout(uint32_t ticks, uint64_t seed, bool harmless, unsigned simpleMask)
 {
     check(pom_batch_rollout(handle, ticks, seed, tick, (harmless ? POM_ROLL_HARMLESS : 0) | POM_ROLL_SIMPLE(simpleMask)), "pom_batch_rollout");
