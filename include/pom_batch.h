@@ -205,6 +205,31 @@ typedef struct pom_step_compact_io {
     int32_t         obs_view;
 } pom_step_compact_io;
 int  pom_batch_step_compact(pom_batch* b, const pom_step_compact_io* io, uint32_t flags);
+/* pom_batch_step that also writes every env's per-agent REWARD of this tick, from inside the step kernel, for a learning
+ * loop that keeps everything on the device (pom_batch_policy_moves -> pom_batch_step_rewards -> pom_batch_observe_planes).
+ *   moves_dev  as for pom_batch_step
+ *   rewards    n_envs x 4 int8 (4-byte aligned), required: byte a of env e at 4 e + a is the reward r[a] of agent a
+ *   status     n_envs bytes or NULL: the end-of-tick status byte before any auto-reset, as pom_batch_step_host's status_host
+ * Every env gets its four values, zeros included.  The reference has no reward; this is the project's definition, after the
+ * reward function of the Pommerman Python environment.  With `stepped` = the env had neither DONE nor INVALID when the
+ * tick started, `st` = its status byte as reported in `status`, and dead[a] = agent a's dead flag after the tick, the
+ * first matching case decides:
+ *     case                        free-for-all                      team game (POM_INIT_TEAMS)
+ *     not stepped                 0 0 0 0                           0 0 0 0
+ *     st & INVALID                0 0 0 0 (aborted, no outcome)     0 0 0 0
+ *     DONE, not DRAW, winner w    +1 for agent w, -1 for the rest   +1 for both agents of team w, -1 for the other two
+ *     DONE | DRAW                 -1 -1 -1 -1                       -1 -1 -1 -1
+ *     TRUNCATED                   -1 -1 -1 -1                       -1 -1 -1 -1
+ *     running                     -1 if dead[a], else 0             0 0 0 0
+ * TRUNCATED is set only when DONE is not, so a win on the last allowed tick is a win.  In free-for-all a dead agent
+ * collects -1 on every tick until its episode ends, the terminal tick included; a caller that wants a single -1 at death
+ * takes the first one.  Frozen envs (done or invalid without POM_STEP_AUTORESET) get zeros.
+ * Each pointer may be device memory or page-locked mapped host memory (pom_host_alloc).  Accepted flags: POM_STEP_AUTORESET,
+ * POM_STEP_COUNT, POM_STEP_CONTINUE_UNDEFINED; states, counters, episode numbers and resets are those of pom_batch_step
+ * with the same moves.  POM_E_ARG for any other flag (POM_STEP_RAW keeps no episode, so there is no outcome), a null
+ * rewards, pageable buffers, or a handle made with POM_STEP_KERNEL=tile.  Enqueues only: results are valid after
+ * pom_batch_sync(b). */
+int  pom_batch_step_rewards(pom_batch* b, const uint8_t* moves_dev, uint32_t flags, int8_t* rewards, uint8_t* status);
 /* `ticks` fused ticks with the boards resident in shared memory; actions from pom_rng_moves(rng_seed,
  * global env index, tick0 + k); auto-reset unless POM_ROLL_NO_RESET.  Replaces the loop of
  * Environment::StartGame (environment.cpp:68-88) with RandomAgent/HarmlessAgent::act (bboard.hpp:517-533), or with

@@ -256,6 +256,9 @@ public:
      * (simple_agent.cpp:12-141; their draws come from the shared counter RNG keyed by `seed`) and the others
      * take their move from `moves` (n x 4, host memory; entries of masked agents are ignored) */
     size_t Step(const Move* moves, unsigned simpleMask, uint64_t seed);
+    /* Step(moves) that also fills rewards (n x 4, host memory) with every game's per-agent reward of this tick:
+     * rewards[4 * i + a] for agent a of game i, as pom_batch_step_rewards defines it (include/pom_batch.h) */
+    size_t Step(const Move* moves, int8_t* rewards);
     /* `ticks` ticks in ONE launch with the given moves (ticks x n x 4, tick-major, host memory); finished games freeze.
      * Returns the number of games still running.  For replaying traces and evaluating fixed action plans. */
     size_t StepSequence(const Move* moves, uint32_t ticks);

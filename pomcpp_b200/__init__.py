@@ -148,6 +148,7 @@ def lib():
         L.pom_bind_thread_near.argtypes = [i32]
         L.pom_batch_step_compact.argtypes = [vp, vp, u32]
         L.pom_batch_step_observe.argtypes = [vp, vp, u32, vp, u32, i32]
+        L.pom_batch_step_rewards.argtypes = [vp, vp, u32, vp, vp]
         L.pom_batch_event_record.argtypes = [vp, i32]
         L.pom_batch_event_elapsed_ms.argtypes = [vp, C.POINTER(C.c_float)]
         L.pom_batch_flush_l2.argtypes = [vp]
@@ -321,6 +322,14 @@ class Batch:
                            0 if fin_env is None else (fin_env.size if hasattr(fin_env, "size") else self.n),
                            obs_dev, obs_agent_mask, obs_view)
         _ck(lib().pom_batch_step_compact(self.h, C.byref(io), flags))
+
+    def step_rewards(self, moves_dev, rewards, status=None, flags=0):
+        """one tick that also writes every env's four int8 rewards (pom_batch_step_rewards): `rewards` = n x 4 bytes,
+        `status` = n status bytes (optional), as pom_batch_step_host reports them.  Arrays must live in pinned mapped memory
+        (pinned_array) or be raw device pointers; enqueue only."""
+        def ptr(a):
+            return a if isinstance(a, (int, C.c_void_p)) else _p(a)
+        _ck(lib().pom_batch_step_rewards(self.h, ptr(moves_dev), flags, ptr(rewards), ptr(status)))
 
     def step_seq(self, moves_dev, ticks, flags=0):
         """`ticks` ticks in one launch with the caller's moves (device pointer, ticks x n x 4 bytes, tick-major)"""

@@ -246,31 +246,39 @@ int pack_into(pom_batch* b, uint8_t* dst_recs, uint64_t first, uint64_t count, c
 /* geometry of the persistent per-tick kernel (k_step_ws): compute warps and slice buffers per CTA (= per SM) */
 constexpr int WS_NW = 20, WS_NBUF = 24;
 
-template<int NW, bool OBS, bool FREEZE = false, bool SPEC = false, bool TEAMS = false>
+template<int NW, bool OBS, bool FREEZE = false, bool SPEC = false, bool TEAMS = false, bool REWARDS = false>
 int launch_step_ws(pom_batch* b, const pomk::BatchParams& P, const pomk::StepIO& io, uint32_t flags, cudaStream_t on)
 {
     typedef pomk::RingScratch<WS_NBUF> R;
-    /* NW is even and >= 12; the team images (NW = WS_NW only) take bits 24..26 */
-    const uint32_t bit = TEAMS ? (1u << (24 + (FREEZE ? 2 : (OBS ? 1 : 0)))) :
+    /* NW is even and >= 12; the team images (NW = WS_NW only) take bits 24..26, the REWARDS images bits 27..28 */
+    const uint32_t bit = REWARDS ? (1u << (TEAMS ? 28 : 27)) :
+                         TEAMS ? (1u << (24 + (FREEZE ? 2 : (OBS ? 1 : 0)))) :
                          SPEC ? 2u : (FREEZE ? 1u : (1u << (NW + (OBS ? 1 : 0))));
     if(!(b->attr_ws & bit))
     {
-        CK(cudaFuncSetAttribute(pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC, TEAMS>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(R::BYTES)));
+        CK(cudaFuncSetAttribute(pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC, TEAMS, REWARDS>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(R::BYTES)));
         b->attr_ws |= bit;
     }
     const uint64_t n_slices = (P.n_envs + 31) / 32;
     const unsigned grid = unsigned(n_slices < uint64_t(b->n_sms) ? n_slices : uint64_t(b->n_sms));
-    pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC, TEAMS><<<grid, (NW + 1) * 32, R::BYTES, on ? on : b->stream>>>(P, io, flags);
+    pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC, TEAMS, REWARDS><<<grid, (NW + 1) * 32, R::BYTES, on ? on : b->stream>>>(P, io, flags);
     b->launches++;
     CK(cudaGetLastError());
     return POM_OK;
 }
 
-int launch_step_io(pom_batch* b, const pomk::BatchParams& P, pomk::StepIO io, uint32_t flags, cudaStream_t on)
+/* rewards: pom_batch_step_rewards, whose output travels in io.obs, so this is decided first */
+int launch_step_io(pom_batch* b, const pomk::BatchParams& P, pomk::StepIO io, uint32_t flags, cudaStream_t on, bool rewards = false)
 {
     io.bulk = (reinterpret_cast<uintptr_t>(io.moves) & 15u) == 0u ? 1u : 0u;   /* TMA needs 16-byte alignment */
     /* whole-batch launches alternate the direction of the walk (L2 reuse between ticks, see StepIO::reverse) */
     if(P.n_envs == b->n_envs && b->pingpong) io.reverse = (b->walk++) & 1u;
+    /* the REWARDS images exist for the default geometry and the generic image only (no SPEC, no POM_WS_NW variants) */
+    if(rewards)
+    {
+        if(b->teams) return launch_step_ws<WS_NW, false, false, false, true, true>(b, P, io, flags, on);
+        return launch_step_ws<WS_NW, false, false, false, false, true>(b, P, io, flags, on);
+    }
     if(b->teams)
     {
         /* the team game has the generic images of the default geometry only: no SPEC image, no POM_WS_NW variants */
@@ -888,6 +896,26 @@ int pom_batch_step_compact(pom_batch* b, const pom_step_compact_io* io, uint32_t
     rc = launch_step_io(b, b->params(), k, flags, b->stream);
     if(rc || !io->obs_dev || b->obs_fused) return rc;
     POM_DISPATCH(b, launch_observe_planes, b, io->obs_dev, io->obs_agent_mask, io->obs_view);
+}
+
+int pom_batch_step_rewards(pom_batch* b, const uint8_t* moves_dev, uint32_t flags, int8_t* rewards, uint8_t* status)
+{
+    int rc = use(b); if(rc) return rc;
+    if(!moves_dev || !rewards) return fail(POM_E_ARG, "pom_batch_step_rewards: null moves or rewards");
+    if(flags & ~uint32_t(POM_STEP_AUTORESET | POM_STEP_COUNT | POM_STEP_CONTINUE_UNDEFINED))
+        return fail(POM_E_ARG, "pom_batch_step_rewards: only POM_STEP_AUTORESET, POM_STEP_COUNT and POM_STEP_CONTINUE_UNDEFINED are accepted");
+    if(b->step_kernel != 0) return fail(POM_E_ARG, "pom_batch_step_rewards needs the persistent step kernel (unset POM_STEP_KERNEL)");
+    pomk::StepIO k{};
+    uint8_t* moves = nullptr; int8_t* rw = nullptr;
+    const char* bad = "pom_batch_step_rewards: buffers must be device memory or page-locked mapped host memory (pom_host_alloc)";
+    if((rc = device_view(const_cast<uint8_t*>(moves_dev), &moves, bad))) return rc;
+    if((rc = device_view(rewards, &rw, bad))) return rc;
+    if((rc = device_view(status, &k.status_out, bad))) return rc;
+    /* each env's four rewards are stored as one word */
+    if(reinterpret_cast<uintptr_t>(rw) & 3u) return fail(POM_E_ARG, "pom_batch_step_rewards: rewards must be 4-byte aligned");
+    k.moves = moves;
+    k.obs = reinterpret_cast<uint8_t*>(rw);                           /* the REWARDS images' output slot (StepIO::obs) */
+    return launch_step_io(b, b->params(), k, flags, b->stream, true);
 }
 
 int pom_batch_rollout(pom_batch* b, uint32_t ticks, uint64_t rng_seed, uint32_t tick0, uint32_t flags)

@@ -1377,6 +1377,31 @@ POM_HD int env_step(uint8_t* r, uint32_t moves, int invalid_mask = F_INVALID_MAS
     return flags;
 }
 
+/* The per-agent reward of one tick (pom_batch_step_rewards; the reference has no reward, so this is the project's
+ * definition, after the reward function of the Pommerman Python environment).  Byte a of the result is r[a] as an int8:
+ *   not stepped (the env was done or invalid when the tick started)   0 for everyone
+ *   st & INVALID                                                       0 for everyone (aborted episode, no outcome)
+ *   DONE, winner w                        +1 for w (team game: both agents of team w), -1 for the others
+ *   DONE | DRAW, or TRUNCATED                                         -1 for everyone
+ *   running        free-for-all: -1 for a dead agent, 0 for a live one; team game: 0 for everyone
+ * `st` is the end-of-tick status byte BEFORE any auto-reset (what status_out reports); `aflags` the record's agent-flags
+ * word after the tick.  TRUNCATED is only set when DONE is not, so a win on the last allowed tick is a win.  aflags is
+ * read only while the game runs, and a running env is never reset: the word may come from the record after the reset. */
+template<bool TEAMS = false>
+POM_HD uint32_t tick_rewards(bool stepped, uint32_t st, uint32_t aflags)
+{
+    if(!stepped || (st & POM_STATUS_INVALID)) return 0u;
+    if((st & (POM_STATUS_DONE | POM_STATUS_DRAW)) == POM_STATUS_DONE)
+    {
+        const uint32_t w = (st & POM_STATUS_WINNER_MASK) >> POM_STATUS_WINNER_SHIFT;
+        const uint32_t win = TEAMS ? (0x00FF00FFu << (8u * (w & 1u))) : (0xFFu << (8u * w));
+        return (0xFFFFFFFFu & ~win) | (0x01010101u & win);
+    }
+    if(st & (POM_STATUS_DONE | POM_STATUS_TRUNCATED)) return 0xFFFFFFFFu;
+    if(TEAMS) return 0u;
+    return ((aflags >> 1) & 0x01010101u) * 0xFFu;                    /* AF_DEAD = bit 1 of each agent's byte */
+}
+
 /* ---------------------------------------------------------------------------------------------
  * AoS <-> record converters (K5).  pack() returns 0, or a non-zero reason when the AoS state holds
  * a value the record cannot carry (the env is then marked POM_STATUS_INVALID).

@@ -491,11 +491,16 @@ struct StepIO {
     uint32_t    fin_capacity;
     uint8_t*    obs;           /* observation planes of the agents in obs_mask, written from the resident record at the
                                   end of the tick (after an auto-reset): slab k (k-th agent of the mask) at
-                                  obs + k * obs_stride * POM_OBS_BYTES; null = none */
+                                  obs + k * obs_stride * POM_OBS_BYTES; null = none.
+                                  The REWARDS images, which are OBS = false images, take their output here instead:
+                                  one word per env, byte a = the int8 reward of agent a (pomcore::tick_rewards).  The slot
+                                  keeps its one type: a union with a uint32_t* changed the SASS of the OBS images. */
     uint64_t    obs_stride;
     uint32_t    obs_mask;
     int         obs_view;
 };
+/* the kernel-parameter size is part of every k_step_ws image: a new output shares a slot instead of growing the struct */
+static_assert(sizeof(StepIO) == 104, "StepIO changes the parameter block of every k_step_ws image");
 
 /* four moves from a joint action index */
 __device__ __forceinline__ uint32_t moves_of_joint(uint32_t j)
@@ -531,7 +536,10 @@ template<int NBUF> struct RingScratch {
  * the two-stream overlap).  The same treatment of the compact-I/O configuration was measured 6-15 % SLOWER than the
  * generic image in three variants (all of io constant; the flags only; joint + bulk only) and is not built: what the
  * compiler makes of this loop body is not monotone in what it knows (see also FREEZE below). */
-template<int NW, int NBUF, bool OBS, bool FREEZE, bool SPEC = false, bool TEAMS = false>
+/* REWARDS: the image of pom_batch_step_rewards - every active env also stores its four int8 rewards (pomcore::tick_rewards)
+ * as one word to the array in StepIO::obs, next to its status byte.  Its own image for the reason FREEZE and TEAMS have theirs:
+ * the plain step keeps its code as it is. */
+template<int NW, int NBUF, bool OBS, bool FREEZE, bool SPEC = false, bool TEAMS = false, bool REWARDS = false>
 __global__ void __launch_bounds__((NW + 1) * 32, 1) k_step_ws(BatchParams P, StepIO io_in, uint32_t flags_in)
 {
     const uint32_t flags = SPEC ? uint32_t(POM_STEP_AUTORESET | POM_STEP_COUNT) : flags_in;
@@ -641,6 +649,9 @@ __global__ void __launch_bounds__((NW + 1) * 32, 1) k_step_ws(BatchParams P, Ste
             if(active && stepped) st_end = st;
         }
         if(status_out && active) status_out[env] = uint8_t(st_end);
+        /* after a reset the record is the template's, but tick_rewards reads the agent flags only while the game runs */
+        if(REWARDS && active)
+            reinterpret_cast<uint32_t*>(io.obs)[env] = pomcore::tick_rewards<TEAMS>(stepped, st_end, *reinterpret_cast<const uint32_t*>(rec + R_AFLAGS));
         if(io.done_bits || io.fin_env)
         {
             /* compact results: which envs ended an episode in this tick, as one bit per env and as a list */

@@ -391,6 +391,31 @@ size_t BatchEnvironment::Step(const Move* moves, unsigned simpleMask, uint64_t s
     return running;
 }
 
+size_t BatchEnvironment::Step(const Move* moves, int8_t* rewards)
+{
+    /* one pinned buffer the kernel reads and writes directly: moves, rewards, status bytes */
+    void* pinned = nullptr;
+    check(pom_host_alloc(9 * n, &pinned), "pom_host_alloc");
+    uint8_t* mv = static_cast<uint8_t*>(pinned);
+    int8_t* rw = reinterpret_cast<int8_t*>(mv + 4 * n);
+    uint8_t* st = mv + 8 * n;
+    for(size_t i = 0; i < 4 * n; i++) mv[i] = uint8_t(int(moves[i]));
+    int rc = pom_batch_step_rewards(handle, mv, 0, rw, st);
+    if(rc == POM_OK) rc = pom_batch_sync(handle);
+    if(rc == POM_OK)
+    {
+        std::memcpy(rewards, rw, 4 * n);
+        status.assign(st, st + n);
+    }
+    pom_host_free(pinned);
+    check(rc, "pom_batch_step_rewards");
+    fresh = false;
+    tick++;
+    size_t running = 0;
+    for(size_t i = 0; i < n; i++) running += (status[i] & (POM_STATUS_DONE | POM_STATUS_INVALID)) ? 0 : 1;
+    return running;
+}
+
 size_t BatchEnvironment::StepSequence(const Move* moves, uint32_t ticks)
 {
     const size_t bytes = size_t(ticks) * n * 4;
