@@ -87,12 +87,17 @@ typedef struct pom_init_desc {
 
 enum {
     POM_INIT_EMPTY = 0x1,  /* do not fill the envs (they will be uploaded); the pool is still built */
-    POM_INIT_TEAMS = 0x2   /* the handle plays the 2v2 TEAM game: team 0 = agents 0 and 2, team 1 = agents 1 and 3.
+    POM_INIT_TEAMS = 0x2,  /* the handle plays the 2v2 TEAM game: team 0 = agents 0 and 2, team 1 = agents 1 and 3.
                               Step (bboard::Step) is the same, flames kill teammates too; what changes is when an episode
                               ends and who won (pom_state.h: the status byte) and whom the device SimpleAgent treats as an
                               enemy (not its teammate).  The reference has no team mode: this is the project's definition.
                               The mode is fixed for the handle's life and applies to every entry point that steps or acts;
                               pom_batch_clone / pom_batch_expand_step between handles of different modes fail (POM_E_ARG). */
+    POM_INIT_RADIO = 0x4   /* the team game with the TEAM RADIO of Pommerman's team-radio environment (pommerman/envs/v2.py, the
+                              NeurIPS 2018 competition format): every tick each agent sends its teammate two words of 0..7,
+                              which the teammate reads in its next observation (pom_batch_step_radio).  Needs POM_INIT_TEAMS
+                              (POM_E_ARG otherwise); fixed for the handle's life.  pom_batch_clone / pom_batch_expand_step
+                              between a radio and a non-radio handle fail (POM_E_ARG). */
 };
 
 /* episode counters accumulated on the device (Environment::IsDone/IsDraw/GetWinner, bboard.hpp:617-631) */
@@ -116,6 +121,8 @@ int  pom_batch_sync(pom_batch* b);
 const char* pom_last_error(void);
 /* 1 if the handle plays the team game (POM_INIT_TEAMS), 0 for free-for-all, POM_E_ARG for a null handle */
 int  pom_batch_teams(const pom_batch* b);
+/* 1 if the handle has the team radio (POM_INIT_RADIO), 0 if not, POM_E_ARG for a null handle */
+int  pom_batch_radio(const pom_batch* b);
 
 /* ---- AoS <-> packed exchange (there is no reference call: State is passed by pointer) ---- */
 int  pom_batch_upload(pom_batch* b, uint64_t first, uint64_t count, const pom_state* states, const uint8_t* status /* may be NULL */);
@@ -137,6 +144,7 @@ int  pom_batch_observe(pom_batch* b, uint64_t first, uint64_t count, int agent, 
  *   363..483   ticks the visible flame on the cell still burns (timeLeft of its flame-queue entry)
  *   484 x  485 y  486 ammo = maxBombCount - bombCount (clamped to 0..255)  487 blast strength  488 can kick
  *   489 alive mask (bit i = agent i alive; public)  490..491 timeStep (little endian)  492 observer alive  493..511 zero
+ *   (on a radio handle, POM_INIT_RADIO: 493 = w0 and 494 = w1 of the teammate's last message, pom_batch_step_radio)
  * Cells outside the window hold 5 (fog) in the board plane and 0 elsewhere.
  * obs_dev: DEVICE buffer of popcount(agent_mask) slabs of pom_batch_obs_stride(b) observations each; the observation of
  * env e for the k-th agent of the mask (in agent order) starts at ((k * stride) + e) * POM_OBS_BYTES.  The stride is
@@ -149,7 +157,8 @@ int  pom_batch_observe_planes(pom_batch* b, uint8_t* obs_dev, uint32_t agent_mas
  *     p * W * W + row * W + col   plane p (0 board ids, 1 blast strength, 2 bomb timer, 3 flame life, as above) of board
  *                                 cell (x - view + col, y - view + row), (x, y) = the observer's position; window cells
  *                                 that lie off the board hold 5 (fog) in the board plane and 0 elsewhere
- *     4 * W * W ... + 11          the twelve scalar bytes 484..495 of the full layout, then zero padding
+ *     4 * W * W ... + 11          the twelve scalar bytes 484..495 of the full layout, then zero padding (so on a radio
+ *                                 handle the teammate's message is in bytes 4 W W + 9 and 4 W W + 10)
  * Slabs as for pom_batch_observe_planes, with pom_obs_cropped_bytes(view) in place of POM_OBS_BYTES. */
 uint32_t pom_obs_cropped_bytes(int view);   /* 0 for a view outside 0..5 */
 int  pom_batch_observe_planes_cropped(pom_batch* b, uint8_t* obs_dev, uint32_t agent_mask, int view);
@@ -230,6 +239,40 @@ int  pom_batch_step_compact(pom_batch* b, const pom_step_compact_io* io, uint32_
  * rewards, pageable buffers, or a handle made with POM_STEP_KERNEL=tile.  Enqueues only: results are valid after
  * pom_batch_sync(b). */
 int  pom_batch_step_rewards(pom_batch* b, const uint8_t* moves_dev, uint32_t flags, int8_t* rewards, uint8_t* status);
+/* The tick of pom_batch_step_rewards with the TEAM RADIO, on a handle made with POM_INIT_RADIO (POM_E_ARG otherwise).  The
+ * reference has no radio; this is the project's definition, after Pommerman's team-radio environment (action space
+ * Tuple(Discrete(6), Discrete(8), Discrete(8)): a move and two words).
+ *   moves_dev  as for pom_batch_step
+ *   msgs       n_envs x 4 bytes (4-byte aligned): byte a of env e at 4 e + a is agent a's message w0 | w1 << 3, two words
+ *              w0, w1 of 0..7; bits 6..7 are ignored (as a joint action >= 1296 is taken modulo 6 per digit)
+ *   rewards    n_envs x 4 int8 (4-byte aligned) or NULL, status  n_envs bytes or NULL: those of pom_batch_step_rewards
+ * Each env keeps one LAST MESSAGE per agent (initially (0, 0)), in the record's padding bytes (pom_record.h), so the radio
+ * moves no byte of state beyond the record.  Per env, together with its tick:
+ *   not stepped (DONE or INVALID when the tick starts)   the messages stay as they are
+ *   stepped      agent a's last message becomes msgs[4 e + a] & 63 if a was alive when the tick started, (0, 0) if it
+ *                was dead (Pommerman's `not agent.is_alive` check before stepping): an agent that dies in this tick
+ *                still gets its message through
+ *   the env ended this tick and POM_STEP_AUTORESET re-initialised it: (0, 0) for everyone in the new episode
+ * States, status bytes, counters and rewards are exactly those of pom_batch_step_rewards with the same moves: the radio
+ * never changes the game.  Accepted flags: POM_STEP_AUTORESET, POM_STEP_COUNT, POM_STEP_CONTINUE_UNDEFINED.  POM_E_ARG for
+ * any other flag, null moves or msgs, pageable buffers, misaligned msgs or rewards, or a handle made with
+ * POM_STEP_KERNEL=tile.  Enqueues only: results are valid after pom_batch_sync(b).
+ * Messages are env state, like the record.  Only this call, pom_batch_radio_upload and (re-)initialisation change them;
+ * (re-)initialisation (auto-reset in any stepping path, pom_batch_reset, pom_batch_upload) sets (0, 0).  Every other call
+ * - pom_batch_step[_host|_compact|_seq|_observe], pom_batch_rollout, pom_batch_policy_* - leaves the messages of running
+ * envs as they were; pom_batch_clone copies them and pom_batch_expand_step children inherit their root's.  (Pommerman
+ * sends (0, 0) for an action without words; here a step without messages keeps the last ones, which leaves every other
+ * kernel as it is.)
+ * The observation planes of a radio handle carry, for observer a, the last message of its teammate a ^ 2: byte 493 = w0
+ * and byte 494 = w1 in the full layout, scalar bytes 9 and 10 in the cropped one (zero on every other handle); the radio
+ * is not fogged.  This holds for pom_batch_observe_planes[_cropped], pom_batch_step_observe and pom_step_compact_io's
+ * obs_dev; on a radio handle the last two always queue the observation kernel behind the step (POM_OBS_FUSED does not
+ * apply).  pom_batch_observe (pom_state has no field for it) and the device SimpleAgent ignore the radio. */
+int  pom_batch_step_radio(pom_batch* b, const uint8_t* moves_dev, const uint8_t* msgs, uint32_t flags, int8_t* rewards, uint8_t* status);
+/* last messages of envs [first, first + count) of a radio handle (POM_E_ARG otherwise), count x 4 bytes of HOST memory in
+ * the msgs encoding of pom_batch_step_radio; the upload ignores bits 6..7.  For fixtures, tree-search bookkeeping, tests. */
+int  pom_batch_radio_download(pom_batch* b, uint64_t first, uint64_t count, uint8_t* msgs_host);
+int  pom_batch_radio_upload(pom_batch* b, uint64_t first, uint64_t count, const uint8_t* msgs_host);
 /* `ticks` fused ticks with the boards resident in shared memory; actions from pom_rng_moves(rng_seed,
  * global env index, tick0 + k); auto-reset unless POM_ROLL_NO_RESET.  Replaces the loop of
  * Environment::StartGame (environment.cpp:68-88) with RandomAgent/HarmlessAgent::act (bboard.hpp:517-533), or with

@@ -29,6 +29,7 @@
 #include <functional>
 #include <iostream>
 #include <memory>
+#include <utility>
 #include <vector>
 
 #include "pom_batch.h"
@@ -237,9 +238,10 @@ private:
 class BatchEnvironment
 {
 public:
-    /* teams: the games are 2v2 team games (POM_INIT_TEAMS, include/pom_batch.h: agents 0 and 2 against 1 and 3) */
+    /* teams: the games are 2v2 team games (POM_INIT_TEAMS, include/pom_batch.h: agents 0 and 2 against 1 and 3);
+     * radio: team games with the team radio (POM_INIT_RADIO, needs teams) */
     BatchEnvironment(size_t nGames, int device = 0, uint64_t envOffset = 0, uint32_t nTemplates = 1024,
-                     int firstSeed = 0x1337, uint32_t maxTicks = 0, bool teams = false);
+                     int firstSeed = 0x1337, uint32_t maxTicks = 0, bool teams = false, bool radio = false);
     ~BatchEnvironment();
     BatchEnvironment(const BatchEnvironment&) = delete;
     BatchEnvironment& operator=(const BatchEnvironment&) = delete;
@@ -259,6 +261,12 @@ public:
     /* Step(moves) that also fills rewards (n x 4, host memory) with every game's per-agent reward of this tick:
      * rewards[4 * i + a] for agent a of game i, as pom_batch_step_rewards defines it (include/pom_batch.h) */
     size_t Step(const Move* moves, int8_t* rewards);
+    /* Step(moves, rewards) with the team radio (pom_batch_step_radio; radio games only): messages = n x 4 bytes of host
+     * memory, messages[4 * i + a] = w0 | w1 << 3 for the two words agent a of game i sends its teammate; rewards may be
+     * null.  A name of its own, so that a null rewards pointer cannot pick another overload. */
+    size_t StepRadio(const Move* moves, const uint8_t* messages, int8_t* rewards = nullptr);
+    /* the last message of `agent` in game i, as the words (w0, w1): what its teammate reads in its next observation */
+    std::pair<int, int> GetMessage(size_t i, int agent);
     /* `ticks` ticks in ONE launch with the given moves (ticks x n x 4, tick-major, host memory); finished games freeze.
      * Returns the number of games still running.  For replaying traces and evaluating fixed action plans. */
     size_t StepSequence(const Move* moves, uint32_t ticks);
@@ -283,6 +291,7 @@ public:
     bool IsDraw(size_t i);
     int GetWinner(size_t i);                       /* the winning agent; -1 while running, on a draw and in a team game */
     bool IsTeamGame() const { return teams; }
+    bool HasRadio() const { return radio; }
     int GetWinningTeam(size_t i);                  /* team game: the winning team (0 or 1); -1 while running, on a draw */
     pom_batch* Handle() const { return handle; }
 
@@ -297,6 +306,7 @@ private:
     uint32_t tick = 0;
     int viewRange = -1;
     bool teams = false;
+    bool radio = false;
 };
 
 }

@@ -27,7 +27,7 @@ def ROLL_SIMPLE(agent_mask):
     return (agent_mask & 0xF) << 8
 
 
-INIT_EMPTY, INIT_TEAMS = 1, 2
+INIT_EMPTY, INIT_TEAMS, INIT_RADIO = 1, 2, 4
 
 STATUS_DONE, STATUS_DRAW, STATUS_INVALID, STATUS_TRUNCATED = 0x01, 0x02, 0x10, 0x20
 
@@ -53,6 +53,19 @@ class StepCompactIO(C.Structure):
     _fields_ = [("joint", C.c_void_p), ("done_bits", C.c_void_p), ("fin_env", C.c_void_p), ("fin_status", C.c_void_p),
                 ("fin_count", C.c_void_p), ("fin_capacity", C.c_uint32), ("obs_dev", C.c_void_p),
                 ("obs_agent_mask", C.c_uint32), ("obs_view", C.c_int32)]
+
+
+def pack_messages(words):
+    """[n, 4, 2] radio words (w0, w1 of agent a, each 0..7) -> [n, 4] uint8 in the encoding of pom_batch_step_radio:
+    byte a = w0 | w1 << 3"""
+    w = np.asarray(words, np.uint8).reshape(-1, 4, 2)
+    return ((w[:, :, 0] & 7) | ((w[:, :, 1] & 7) << 3)).astype(np.uint8)
+
+
+def unpack_messages(msgs):
+    """[n, 4] message bytes -> [n, 4, 2] words (w0, w1); bits 6..7 are ignored, as the device ignores them"""
+    m = np.asarray(msgs, np.uint8).reshape(-1, 4)
+    return np.stack([m & 7, (m >> 3) & 7], axis=-1).astype(np.uint8)
 
 
 def joint_of_moves(moves):
@@ -133,6 +146,10 @@ def lib():
         L.pom_batch_generate_moves.argtypes = [vp, vp, u64, u32, u32]
         L.pom_batch_size.restype = u64
         L.pom_batch_teams.argtypes = [vp]
+        L.pom_batch_radio.argtypes = [vp]
+        L.pom_batch_step_radio.argtypes = [vp, vp, vp, u32, vp, vp]
+        L.pom_batch_radio_download.argtypes = [vp, u64, u64, vp]
+        L.pom_batch_radio_upload.argtypes = [vp, u64, u64, vp]
         L.pom_batch_set_policy_view.argtypes = [vp, i32]
         L.pom_batch_get_policy_view.argtypes = [vp, C.POINTER(C.c_int)]
         L.pom_batch_size.argtypes = [vp]
@@ -175,13 +192,13 @@ class Batch:
     """One handle = one shard of envs on one GPU (pom_batch_* of include/pom_batch.h)."""
 
     def __init__(self, n_envs, device=0, env_offset=0, n_templates=1024, first_seed=0x1337,
-                 host_templates=None, max_ticks=0, empty=False, teams=False):
+                 host_templates=None, max_ticks=0, empty=False, teams=False, radio=False):
         self.h = C.c_void_p()
         d = InitDesc()
         d.env_offset = env_offset
         d.first_seed = first_seed
         d.max_ticks = max_ticks
-        d.flags = (INIT_EMPTY if empty else 0) | (INIT_TEAMS if teams else 0)
+        d.flags = (INIT_EMPTY if empty else 0) | (INIT_TEAMS if teams else 0) | (INIT_RADIO if radio else 0)
         self._keep = None
         if host_templates is not None:
             assert host_templates.dtype == STATE_DT
@@ -214,6 +231,24 @@ class Batch:
         r = lib().pom_batch_teams(self.h)
         _ck(min(r, 0))
         return r == 1
+
+    def radio(self):
+        """True if the handle has the team radio (pom_batch_radio; Batch(..., teams=True, radio=True))"""
+        r = lib().pom_batch_radio(self.h)
+        _ck(min(r, 0))
+        return r == 1
+
+    def radio_download(self, first=0, count=None):
+        """[count, 4] uint8: every env's last message per agent, byte a = w0 | w1 << 3 (unpack_messages splits it)"""
+        count = self.n - first if count is None else count
+        m = np.zeros((count, 4), np.uint8)
+        _ck(lib().pom_batch_radio_download(self.h, first, count, _p(m)))
+        return m
+
+    def radio_upload(self, msgs, first=0):
+        """sets the last messages of envs first.. from [count, 4] bytes in the encoding of radio_download"""
+        m = np.ascontiguousarray(msgs, dtype=np.uint8).reshape(-1, 4)
+        _ck(lib().pom_batch_radio_upload(self.h, first, m.shape[0], _p(m)))
 
     def set_policy_view(self, view):
         """fog of war for the device SimpleAgent (pom_batch_set_policy_view): with view >= 0 every later call that runs it
@@ -330,6 +365,14 @@ class Batch:
         def ptr(a):
             return a if isinstance(a, (int, C.c_void_p)) else _p(a)
         _ck(lib().pom_batch_step_rewards(self.h, ptr(moves_dev), flags, ptr(rewards), ptr(status)))
+
+    def step_radio(self, moves_dev, msgs, rewards=None, status=None, flags=0):
+        """one tick of step_rewards with the team radio (pom_batch_step_radio): `msgs` = n x 4 message bytes (pack_messages),
+        `rewards` (n x 4 int8) and `status` (n bytes) optional.  Arrays must live in pinned mapped memory (pinned_array) or be
+        raw device pointers; enqueue only."""
+        def ptr(a):
+            return a if isinstance(a, (int, C.c_void_p)) or a is None else _p(a)
+        _ck(lib().pom_batch_step_radio(self.h, ptr(moves_dev), ptr(msgs), flags, ptr(rewards), ptr(status)))
 
     def step_seq(self, moves_dev, ticks, flags=0):
         """`ticks` ticks in one launch with the caller's moves (device pointer, ticks x n x 4 bytes, tick-major)"""

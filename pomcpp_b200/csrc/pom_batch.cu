@@ -70,6 +70,8 @@ struct pom_batch {
     int       step_kernel = 0;                 /* 0 = k_step_ws (persistent, warp-specialised), 1 = k_step (one CTA per tile); POM_STEP_KERNEL=tile */
     bool      teams = false;                   /* POM_INIT_TEAMS: the 2v2 team game, fixed for the handle's life; every stepping or
                                                   acting launch takes the kernel images of this mode (POM_DISPATCH_MODE) */
+    bool      radio = false;                   /* POM_INIT_RADIO (team game only, fixed for the handle's life): the records' radio bytes
+                                                  hold the team messages; the observation planes take the RADIO images */
     int       policy_view = -1;                /* pom_batch_set_policy_view: >= 0 = the device SimpleAgent plays under fog of war
                                                   with this view (the FOG images, POM_DISPATCH_POLICY), < 0 = on the full state */
     uint8_t*  recs = nullptr;
@@ -98,7 +100,7 @@ struct pom_batch {
     std::vector<int32_t> seeds;
     uint64_t  launches = 0;
     bool      forked = false;                  /* work is pending on s_k2 that the handle's stream has not waited for */
-    uint32_t  attr_done = 0;                   /* kernels whose shared-memory attribute has been set on this handle's device */
+    uint64_t  attr_done = 0;                   /* kernels whose shared-memory attribute has been set on this handle's device */
 
     pomk::BatchParams params() const
     {
@@ -134,6 +136,8 @@ int use(const pom_batch* cb, bool join = true)
 /* The dynamic shared-memory limit of a kernel is a per-device attribute: remember it per handle (one handle = one
  * device), not in a process-wide flag, so that handles on other GPUs and other host threads set it for themselves. */
 enum { ATTR_STEP = 1, ATTR_ROLLOUT = 2, ATTR_ROLLOUT_POLICY = 4, ATTR_POLICY_MOVES = 8, ATTR_EXPAND = 16, ATTR_OBS = 32, ATTR_ROLLOUT_SPEC = 64, ATTR_OBS_CROPPED = 128 };
+/* the RADIO images of k_observe_planes take bits 32 and 33 */
+constexpr uint64_t ATTR_OBS_RADIO = uint64_t(1) << 32, ATTR_OBS_CROPPED_RADIO = uint64_t(1) << 33;
 /* the bit of a kernel's team image, and of its FOG image (bits 16..23 for free-for-all, 24..31 for the team game) */
 constexpr uint32_t attr_bit(uint32_t which, bool teams, bool fog = false) { return (fog ? which << 16 : which) << (teams ? 8 : 0); }
 
@@ -144,7 +148,7 @@ uint32_t policy_view_bits(const pom_batch* b)
 }
 
 template<typename K>
-int set_smem(pom_batch* b, uint32_t which, K kernel, uint32_t bytes)
+int set_smem(pom_batch* b, uint64_t which, K kernel, uint32_t bytes)
 {
     if(b->attr_done & which) return POM_OK;
     CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(bytes)));
@@ -246,34 +250,40 @@ int pack_into(pom_batch* b, uint8_t* dst_recs, uint64_t first, uint64_t count, c
 /* geometry of the persistent per-tick kernel (k_step_ws): compute warps and slice buffers per CTA (= per SM) */
 constexpr int WS_NW = 20, WS_NBUF = 24;
 
-template<int NW, bool OBS, bool FREEZE = false, bool SPEC = false, bool TEAMS = false, bool REWARDS = false>
+template<int NW, bool OBS, bool FREEZE = false, bool SPEC = false, bool TEAMS = false, bool REWARDS = false, bool RADIO = false>
 int launch_step_ws(pom_batch* b, const pomk::BatchParams& P, const pomk::StepIO& io, uint32_t flags, cudaStream_t on)
 {
     typedef pomk::RingScratch<WS_NBUF> R;
-    /* NW is even and >= 12; the team images (NW = WS_NW only) take bits 24..26, the REWARDS images bits 27..28 */
-    const uint32_t bit = REWARDS ? (1u << (TEAMS ? 28 : 27)) :
+    /* NW is even and >= 12; the team images (NW = WS_NW only) take bits 24..26, the REWARDS images bits 27..28, the RADIO
+     * image bit 29 */
+    const uint32_t bit = RADIO ? (1u << 29) :
+                         REWARDS ? (1u << (TEAMS ? 28 : 27)) :
                          TEAMS ? (1u << (24 + (FREEZE ? 2 : (OBS ? 1 : 0)))) :
                          SPEC ? 2u : (FREEZE ? 1u : (1u << (NW + (OBS ? 1 : 0))));
     if(!(b->attr_ws & bit))
     {
-        CK(cudaFuncSetAttribute(pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC, TEAMS, REWARDS>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(R::BYTES)));
+        CK(cudaFuncSetAttribute(pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC, TEAMS, REWARDS, RADIO>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(R::BYTES)));
         b->attr_ws |= bit;
     }
     const uint64_t n_slices = (P.n_envs + 31) / 32;
     const unsigned grid = unsigned(n_slices < uint64_t(b->n_sms) ? n_slices : uint64_t(b->n_sms));
-    pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC, TEAMS, REWARDS><<<grid, (NW + 1) * 32, R::BYTES, on ? on : b->stream>>>(P, io, flags);
+    pomk::k_step_ws<NW, WS_NBUF, OBS, FREEZE, SPEC, TEAMS, REWARDS, RADIO><<<grid, (NW + 1) * 32, R::BYTES, on ? on : b->stream>>>(P, io, flags);
     b->launches++;
     CK(cudaGetLastError());
     return POM_OK;
 }
 
-/* rewards: pom_batch_step_rewards, whose output travels in io.obs, so this is decided first */
-int launch_step_io(pom_batch* b, const pomk::BatchParams& P, pomk::StepIO io, uint32_t flags, cudaStream_t on, bool rewards = false)
+/* rewards: pom_batch_step_rewards, whose output travels in io.obs, so this is decided first; radio: pom_batch_step_radio
+ * (rewards, if any, in io.obs, the messages in io.fin_status) */
+int launch_step_io(pom_batch* b, const pomk::BatchParams& P, pomk::StepIO io, uint32_t flags, cudaStream_t on, bool rewards = false,
+                   bool radio = false)
 {
     io.bulk = (reinterpret_cast<uintptr_t>(io.moves) & 15u) == 0u ? 1u : 0u;   /* TMA needs 16-byte alignment */
     /* whole-batch launches alternate the direction of the walk (L2 reuse between ticks, see StepIO::reverse) */
     if(P.n_envs == b->n_envs && b->pingpong) io.reverse = (b->walk++) & 1u;
-    /* the REWARDS images exist for the default geometry and the generic image only (no SPEC, no POM_WS_NW variants) */
+    /* the REWARDS and RADIO images exist for the default geometry and the generic image only (no SPEC, no POM_WS_NW variants);
+     * the radio is a team-game feature */
+    if(radio) return launch_step_ws<WS_NW, false, false, false, true, true, true>(b, P, io, flags, on);
     if(rewards)
     {
         if(b->teams) return launch_step_ws<WS_NW, false, false, false, true, true>(b, P, io, flags, on);
@@ -371,7 +381,7 @@ int launch_policy_moves(pom_batch* b, uint8_t* moves_dev, uint64_t seed, uint32_
     return POM_OK;
 }
 
-template<int TPB>
+template<int TPB, bool RADIO = false>
 int launch_observe_planes(pom_batch* b, uint8_t* obs_dev, uint32_t mask, int view, uint32_t cropped_bytes = 0)
 {
     const unsigned grid = unsigned((b->n_envs + TPB - 1) / TPB);
@@ -379,13 +389,13 @@ int launch_observe_planes(pom_batch* b, uint8_t* obs_dev, uint32_t mask, int vie
     const uint32_t reverse = (b->pingpong && b->walk && ((b->walk - 1u) & 1u) == 0u) ? 1u : 0u;
     if(cropped_bytes)
     {
-        int rc = set_smem(b, ATTR_OBS_CROPPED, pomk::k_observe_planes<TPB, true>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
-        pomk::k_observe_planes<TPB, true><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), obs_dev, b->n_alloc, mask, view, reverse, cropped_bytes);
+        int rc = set_smem(b, RADIO ? ATTR_OBS_CROPPED_RADIO : ATTR_OBS_CROPPED, pomk::k_observe_planes<TPB, true, RADIO>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
+        pomk::k_observe_planes<TPB, true, RADIO><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), obs_dev, b->n_alloc, mask, view, reverse, cropped_bytes);
     }
     else
     {
-        int rc = set_smem(b, ATTR_OBS, pomk::k_observe_planes<TPB, false>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
-        pomk::k_observe_planes<TPB, false><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), obs_dev, b->n_alloc, mask, view, reverse, 0u);
+        int rc = set_smem(b, RADIO ? ATTR_OBS_RADIO : ATTR_OBS, pomk::k_observe_planes<TPB, false, RADIO>, pomk::TileScratch<TPB>::BYTES); if(rc) return rc;
+        pomk::k_observe_planes<TPB, false, RADIO><<<grid, TPB, pomk::TileScratch<TPB>::BYTES, b->stream>>>(b->params(), obs_dev, b->n_alloc, mask, view, reverse, 0u);
     }
     b->launches++;
     CK(cudaGetLastError());
@@ -477,6 +487,14 @@ bool local_cpus(int device, cpu_set_t* set)
         POM_DISPATCH_MODE(h, fn, __VA_ARGS__); \
     } while(0)
 
+/* the observation planes of a handle: a radio handle takes the RADIO images, which exist for the default geometry only
+ * (POM_TPB does not apply to it) */
+static int launch_observe(pom_batch* b, uint8_t* obs_dev, uint32_t mask, int view, uint32_t cropped_bytes = 0)
+{
+    if(b->radio) return launch_observe_planes<128, true>(b, obs_dev, mask, view, cropped_bytes);
+    POM_DISPATCH(b, launch_observe_planes, b, obs_dev, mask, view, cropped_bytes);
+}
+
 extern "C" {
 
 const char* pom_last_error(void) { return g_err.c_str(); }
@@ -492,6 +510,8 @@ int pom_batch_init(pom_batch** out, int device, uint64_t n_envs, const pom_init_
 {
     if(!out || !desc || n_envs == 0 || desc->n_templates == 0) return fail(POM_E_ARG, "pom_batch_init: bad argument");
     if(n_envs > (uint64_t(1) << 31)) return fail(POM_E_ARG, "pom_batch_init: too many envs for one handle");
+    if((desc->flags & POM_INIT_RADIO) && !(desc->flags & POM_INIT_TEAMS))
+        return fail(POM_E_ARG, "pom_batch_init: POM_INIT_RADIO needs POM_INIT_TEAMS (the radio talks to a teammate)");
     int ndev = 0;
     cudaError_t ce = cudaGetDeviceCount(&ndev);
     if(ce != cudaSuccess || ndev == 0) return fail(POM_E_CUDA, "no CUDA device: the step path has no CPU fallback", ce);
@@ -506,6 +526,7 @@ int pom_batch_init(pom_batch** out, int device, uint64_t n_envs, const pom_init_
     b->n_templates = desc->n_templates;
     b->max_ticks = desc->max_ticks;
     b->teams = (desc->flags & POM_INIT_TEAMS) != 0;
+    b->radio = (desc->flags & POM_INIT_RADIO) != 0;
     cudaDeviceGetAttribute(&b->n_sms, cudaDevAttrMultiProcessorCount, device);
     if(b->n_sms < 1) b->n_sms = 1;
     if(const char* e = std::getenv("POM_STEP_KERNEL")) b->step_kernel = std::strcmp(e, "tile") == 0 ? 1 : 0;
@@ -652,7 +673,7 @@ int pom_batch_observe_planes(pom_batch* b, uint8_t* obs_dev, uint32_t agent_mask
     int rc = use(b); if(rc) return rc;
     if(!obs_dev) return fail(POM_E_ARG, "pom_batch_observe_planes: null output");
     if(agent_mask == 0 || agent_mask > 0xFu || view < 0) return fail(POM_E_ARG, "pom_batch_observe_planes: agent_mask must be 1..15 and view >= 0");
-    POM_DISPATCH(b, launch_observe_planes, b, obs_dev, agent_mask, view);
+    return launch_observe(b, obs_dev, agent_mask, view);
 }
 
 int pom_device_copy(int device, void* dst, const void* src, uint64_t bytes)
@@ -835,7 +856,7 @@ int pom_batch_observe_planes_cropped(pom_batch* b, uint8_t* obs_dev, uint32_t ag
     int rc = use(b); if(rc) return rc;
     if(!obs_dev) return fail(POM_E_ARG, "pom_batch_observe_planes_cropped: null output");
     if(agent_mask == 0 || agent_mask > 0xFu || view < 0 || view > 5) return fail(POM_E_ARG, "pom_batch_observe_planes_cropped: agent_mask must be 1..15 and view 0..5");
-    POM_DISPATCH(b, launch_observe_planes, b, obs_dev, agent_mask, view, pomcore::obs_cropped_bytes(view));
+    return launch_observe(b, obs_dev, agent_mask, view, pomcore::obs_cropped_bytes(view));
 }
 
 int pom_batch_step_observe(pom_batch* b, const uint8_t* moves_dev, uint32_t flags, uint8_t* obs_dev, uint32_t agent_mask, int view)
@@ -847,7 +868,8 @@ int pom_batch_step_observe(pom_batch* b, const uint8_t* moves_dev, uint32_t flag
     if(b->step_kernel != 0) return fail(POM_E_ARG, "pom_batch_step_observe needs the persistent step kernel (unset POM_STEP_KERNEL)");
     pomk::StepIO k{};
     k.moves = moves_dev;
-    if(b->obs_fused)
+    /* the fused images have no radio: a radio handle always takes the two launches */
+    if(b->obs_fused && !b->radio)
     {
         k.obs = obs_dev; k.obs_stride = b->n_alloc; k.obs_mask = agent_mask; k.obs_view = view;
         return launch_step_io(b, b->params(), k, flags, b->stream);
@@ -857,7 +879,7 @@ int pom_batch_step_observe(pom_batch* b, const uint8_t* moves_dev, uint32_t flag
      * of them per SM no longer cover the latency: 0.267 ms per 1 Mi envs against 0.104 + 0.135 ms (DESIGN section 8). */
     rc = launch_step_io(b, b->params(), k, flags, b->stream);
     if(rc) return rc;
-    POM_DISPATCH(b, launch_observe_planes, b, obs_dev, agent_mask, view);
+    return launch_observe(b, obs_dev, agent_mask, view);
 }
 
 int pom_batch_step_compact(pom_batch* b, const pom_step_compact_io* io, uint32_t flags)
@@ -881,7 +903,7 @@ int pom_batch_step_compact(pom_batch* b, const pom_step_compact_io* io, uint32_t
     if(io->obs_dev)
     {
         if(io->obs_agent_mask == 0 || io->obs_agent_mask > 0xFu || io->obs_view < 0) return fail(POM_E_ARG, "pom_batch_step_compact: obs_agent_mask must be 1..15 and obs_view >= 0");
-        if(b->obs_fused) { k.obs = io->obs_dev; k.obs_stride = b->n_alloc; k.obs_mask = io->obs_agent_mask; k.obs_view = io->obs_view; }
+        if(b->obs_fused && !b->radio) { k.obs = io->obs_dev; k.obs_stride = b->n_alloc; k.obs_mask = io->obs_agent_mask; k.obs_view = io->obs_view; }
     }
     if(k.fin_env)
     {
@@ -894,8 +916,8 @@ int pom_batch_step_compact(pom_batch* b, const pom_step_compact_io* io, uint32_t
         k.fin_count_out = count;
     }
     rc = launch_step_io(b, b->params(), k, flags, b->stream);
-    if(rc || !io->obs_dev || b->obs_fused) return rc;
-    POM_DISPATCH(b, launch_observe_planes, b, io->obs_dev, io->obs_agent_mask, io->obs_view);
+    if(rc || !io->obs_dev || k.obs) return rc;
+    return launch_observe(b, io->obs_dev, io->obs_agent_mask, io->obs_view);
 }
 
 int pom_batch_step_rewards(pom_batch* b, const uint8_t* moves_dev, uint32_t flags, int8_t* rewards, uint8_t* status)
@@ -916,6 +938,30 @@ int pom_batch_step_rewards(pom_batch* b, const uint8_t* moves_dev, uint32_t flag
     k.moves = moves;
     k.obs = reinterpret_cast<uint8_t*>(rw);                           /* the REWARDS images' output slot (StepIO::obs) */
     return launch_step_io(b, b->params(), k, flags, b->stream, true);
+}
+
+int pom_batch_step_radio(pom_batch* b, const uint8_t* moves_dev, const uint8_t* msgs, uint32_t flags, int8_t* rewards, uint8_t* status)
+{
+    int rc = use(b); if(rc) return rc;
+    if(!b->radio) return fail(POM_E_ARG, "pom_batch_step_radio needs a handle made with POM_INIT_RADIO");
+    if(!moves_dev || !msgs) return fail(POM_E_ARG, "pom_batch_step_radio: null moves or messages");
+    if(flags & ~uint32_t(POM_STEP_AUTORESET | POM_STEP_COUNT | POM_STEP_CONTINUE_UNDEFINED))
+        return fail(POM_E_ARG, "pom_batch_step_radio: only POM_STEP_AUTORESET, POM_STEP_COUNT and POM_STEP_CONTINUE_UNDEFINED are accepted");
+    if(b->step_kernel != 0) return fail(POM_E_ARG, "pom_batch_step_radio needs the persistent step kernel (unset POM_STEP_KERNEL)");
+    pomk::StepIO k{};
+    uint8_t* moves = nullptr; uint8_t* m = nullptr; int8_t* rw = nullptr;
+    const char* bad = "pom_batch_step_radio: buffers must be device memory or page-locked mapped host memory (pom_host_alloc)";
+    if((rc = device_view(const_cast<uint8_t*>(moves_dev), &moves, bad))) return rc;
+    if((rc = device_view(const_cast<uint8_t*>(msgs), &m, bad))) return rc;
+    if((rc = device_view(rewards, &rw, bad))) return rc;
+    if((rc = device_view(status, &k.status_out, bad))) return rc;
+    /* each env's four message bytes are loaded, and its four rewards stored, as one word */
+    if((reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(rw)) & 3u)
+        return fail(POM_E_ARG, "pom_batch_step_radio: msgs and rewards must be 4-byte aligned");
+    k.moves = moves;
+    k.obs = reinterpret_cast<uint8_t*>(rw);                           /* the RADIO image's rewards slot (StepIO::obs), may be null */
+    k.fin_status = m;                                                 /* its messages slot (StepIO::fin_status) */
+    return launch_step_io(b, b->params(), k, flags, b->stream, true, true);
 }
 
 int pom_batch_rollout(pom_batch* b, uint32_t ticks, uint64_t rng_seed, uint32_t tick0, uint32_t flags)
@@ -1048,6 +1094,7 @@ int pom_batch_clone(pom_batch* dst, uint64_t first_dst, const pom_batch* src, co
     if(!src || !src_idx) return fail(POM_E_ARG, "pom_batch_clone: null argument");
     if(src->device != dst->device) return fail(POM_E_ARG, "pom_batch_clone: handles live on different devices");
     if(src->teams != dst->teams) return fail(POM_E_ARG, "pom_batch_clone: one handle plays the team game and the other free-for-all (status bytes mean different things)");
+    if(src->radio != dst->radio) return fail(POM_E_ARG, "pom_batch_clone: one handle has the radio and the other not (a record's radio bytes would leak)");
     if(src != dst) { rc = use(src); if(rc) return rc; }         /* joins src's second compute stream if a step is in flight there */
     if(first_dst > dst->n_envs || n_dst > dst->n_envs - first_dst) return fail(POM_E_RANGE, "pom_batch_clone: destination range outside the batch");
     for(uint64_t i = 0; i < n_dst; i++) if(src_idx[i] >= src->n_envs) return fail(POM_E_RANGE, "pom_batch_clone: source index outside the batch");
@@ -1080,6 +1127,7 @@ int pom_batch_expand_step(pom_batch* dst, const pom_batch* src, const uint32_t* 
     if(!src || !src_idx || src == dst) return fail(POM_E_ARG, "pom_batch_expand_step: bad argument");
     if(src->device != dst->device) return fail(POM_E_ARG, "pom_batch_expand_step: handles live on different devices");
     if(src->teams != dst->teams) return fail(POM_E_ARG, "pom_batch_expand_step: one handle plays the team game and the other free-for-all (status bytes mean different things)");
+    if(src->radio != dst->radio) return fail(POM_E_ARG, "pom_batch_expand_step: one handle has the radio and the other not (a record's radio bytes would leak)");
     rc = use(src); if(rc) return rc;                              /* joins src's second compute stream if a step is in flight there */
     if(fanout == 0 || fanout > 1296) return fail(POM_E_ARG, "pom_batch_expand_step: fanout must be 1..1296");
     const uint64_t n_children = n_roots * fanout;
@@ -1203,6 +1251,41 @@ int pom_batch_generate_moves(pom_batch* b, uint8_t* moves_dev, uint64_t seed, ui
 
 uint64_t pom_batch_size(const pom_batch* b) { return b ? b->n_envs : 0; }
 int      pom_batch_teams(const pom_batch* b) { return b ? (b->teams ? 1 : 0) : fail(POM_E_ARG, "pom_batch_teams: null handle"); }
+int      pom_batch_radio(const pom_batch* b) { return b ? (b->radio ? 1 : 0) : fail(POM_E_ARG, "pom_batch_radio: null handle"); }
+
+int pom_batch_radio_download(pom_batch* b, uint64_t first, uint64_t count, uint8_t* msgs_host)
+{
+    int rc = use(b); if(rc) return rc;
+    if(!b->radio) return fail(POM_E_ARG, "pom_batch_radio_download needs a handle made with POM_INIT_RADIO");
+    if(!msgs_host) return fail(POM_E_ARG, "pom_batch_radio_download: null output");
+    if(first > b->n_envs || count > b->n_envs - first) return fail(POM_E_RANGE, "pom_batch_radio_download: range outside the batch");
+    if(!count) return POM_OK;
+    DevBuf buf;
+    CK(buf.alloc(4 * count));
+    pomk::k_radio_download<<<unsigned((count + 127) / 128), 128, 0, b->stream>>>(b->recs, buf.as<uint32_t>(), first, count);
+    b->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(msgs_host, buf.p, 4 * count, cudaMemcpyDeviceToHost, b->stream));
+    CK(cudaStreamSynchronize(b->stream));
+    return POM_OK;
+}
+
+int pom_batch_radio_upload(pom_batch* b, uint64_t first, uint64_t count, const uint8_t* msgs_host)
+{
+    int rc = use(b); if(rc) return rc;
+    if(!b->radio) return fail(POM_E_ARG, "pom_batch_radio_upload needs a handle made with POM_INIT_RADIO");
+    if(!msgs_host) return fail(POM_E_ARG, "pom_batch_radio_upload: null input");
+    if(first > b->n_envs || count > b->n_envs - first) return fail(POM_E_RANGE, "pom_batch_radio_upload: range outside the batch");
+    if(!count) return POM_OK;
+    DevBuf buf;
+    CK(buf.alloc(4 * count));
+    CK(cudaMemcpyAsync(buf.p, msgs_host, 4 * count, cudaMemcpyHostToDevice, b->stream));
+    pomk::k_radio_upload<<<unsigned((count + 127) / 128), 128, 0, b->stream>>>(b->recs, buf.as<uint32_t>(), first, count);
+    b->launches++;
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(b->stream));
+    return POM_OK;
+}
 
 int pom_batch_set_policy_view(pom_batch* b, int view)
 {

@@ -1402,6 +1402,38 @@ POM_HD uint32_t tick_rewards(bool stepped, uint32_t st, uint32_t aflags)
     return ((aflags >> 1) & 0x01010101u) * 0xFFu;                    /* AF_DEAD = bit 1 of each agent's byte */
 }
 
+/* The team radio (POM_INIT_RADIO; after the team-radio environment of Pommerman, pommerman/envs/v2.py).  Record bytes
+ * R_RADIO..R_RADIO + 2, zero padding on every other handle, hold each agent's last message: two words w0, w1 of 0..7 as
+ * the 6-bit value w0 | w1 << 3, agent a in bits 6a..6a+5 of the little-endian 24-bit value. */
+POM_HD uint32_t radio_message(const uint8_t* r, int agent)
+{
+    const uint32_t v = uint32_t(r[R_RADIO]) | (uint32_t(r[R_RADIO + 1]) << 8) | (uint32_t(r[R_RADIO + 2]) << 16);
+    return (v >> (6 * agent)) & 63u;
+}
+
+/* the latch of a tick that steps the env (pom_batch_step_radio): byte a of `msgs` (bits 0..5) becomes agent a's last
+ * message if a's dead flag is clear, (0, 0) if it is set.  Run BEFORE the tick, on the start-of-tick dead flags: an agent
+ * that dies in this tick still gets its message through (Pommerman checks `not agent.is_alive` before stepping).  An
+ * auto-reset after the tick overwrites the bytes with the template's zeros. */
+POM_HD void radio_latch(uint8_t* r, uint32_t msgs)
+{
+    const uint32_t aflags = *reinterpret_cast<const uint32_t*>(r + R_AFLAGS);
+    uint32_t v = 0u;
+    for(int a = 0; a < 4; a++)
+        if(!((aflags >> (8 * a)) & AF_DEAD)) v |= ((msgs >> (8 * a)) & 63u) << (6 * a);
+    r[R_RADIO] = uint8_t(v);
+    r[R_RADIO + 1] = uint8_t(v >> 8);
+    r[R_RADIO + 2] = uint8_t(v >> 16);
+}
+
+/* the scalar word of an observation that holds "observer alive" in its byte 0 gets the teammate's (agent ^ 2) last
+ * message in bytes 1 and 2: w0, then w1 */
+POM_HD uint32_t radio_obs_bytes(const uint8_t* r, int agent)
+{
+    const uint32_t m = radio_message(r, agent ^ 2);
+    return ((m & 7u) << 8) | ((m >> 3) << 16);
+}
+
 /* ---------------------------------------------------------------------------------------------
  * AoS <-> record converters (K5).  pack() returns 0, or a non-zero reason when the AoS state holds
  * a value the record cannot carry (the env is then marked POM_STATUS_INVALID).
@@ -1668,6 +1700,8 @@ POM_HD void obs_cell_coords(int x, int y, uint32_t& xs, uint32_t& ys)
  * 10..13; flame codes have the top bit set -> 4 - then cells outside the window are overwritten with 5, fog), the empty
  * chunks i + 4 and i + 8 of planes 1-3, and chunk i + 12 (part 3: the scalars).  Returns bit w for every board word w
  * of this chunk that shows a visible flame cell. */
+/* RADIO: the observation of a radio handle - bytes 493 and 494 carry the teammate's last message (radio_obs_bytes) */
+template<bool RADIO = false>
 POM_HD uint32_t observe_part_chunks(const uint8_t* r, int agent, const ObsWindow& W, uint8_t* out, int i)
 {
     const uint32_t H = 0x80808080u;
@@ -1714,6 +1748,7 @@ POM_HD uint32_t observe_part_chunks(const uint8_t* r, int agent, const ObsWindow
         s1 = (ap & 15u) | ((ap >> 4) << 8) | (uint32_t(ammo < 0 ? 0 : (ammo > 255 ? 255 : ammo)) << 16) | (uint32_t(r[R_ASTR + agent]) << 24);
         s2 = ((r[R_AFLAGS + agent] & AF_CANKICK) ? 1u : 0u) | (alive << 8) | (uint32_t(r[R_TIME]) << 16) | (uint32_t(r[R_TIME + 1]) << 24);
         s3 = (alive >> agent) & 1u;
+        if(RADIO) s3 |= radio_obs_bytes(r, agent);
     }
     obs_store32(out, i + 12, 0u, s1, s2, s3, 0u, 0u, 0u, 0u);
     return litWords;
@@ -1784,11 +1819,12 @@ POM_HD void observe_part_patches(const uint8_t* r, const ObsWindow& W, uint8_t* 
 }
 
 /* the four parts one after the other (tests/hostsim; not used by the kernels) */
+template<bool RADIO = false>
 POM_HD void observe_planes(const uint8_t* r, int agent, int view, uint8_t* out)
 {
     const ObsWindow W = obs_window(r, agent, view);
     uint32_t lit = 0u;
-    for(int i = 0; i < 4; i++) lit |= observe_part_chunks(r, agent, W, out, i);
+    for(int i = 0; i < 4; i++) lit |= observe_part_chunks<RADIO>(r, agent, W, out, i);
     for(int i = 0; i < 4; i++) observe_part_patches(r, W, out, i, lit);
 }
 
@@ -1807,7 +1843,9 @@ POM_HD uint32_t obs_item_id(uint32_t code)
     return (code & 0x80u) ? 4u : (code >= 8u ? code - 3u : (code == 7u ? 3u : (code >= 2u ? 2u : code)));
 }
 
-/* part i, the chunks.  Returns the mask of this part's board-plane bytes (bit b = byte 32 i + b) that show a flame. */
+/* part i, the chunks.  Returns the mask of this part's board-plane bytes (bit b = byte 32 i + b) that show a flame.
+ * RADIO: scalar bytes 9 and 10 carry the teammate's last message, as bytes 493 and 494 of the full layout. */
+template<bool RADIO = false>
 POM_HD uint32_t observe_cropped_part_chunks(const uint8_t* r, int agent, int view, uint8_t* out, int i)
 {
     const int W = 2 * view + 1, W2 = W * W;
@@ -1825,6 +1863,7 @@ POM_HD uint32_t observe_cropped_part_chunks(const uint8_t* r, int agent, int vie
         sc0 = (ap & 15u) | ((ap >> 4) << 8) | (uint32_t(ammo < 0 ? 0 : (ammo > 255 ? 255 : ammo)) << 16) | (uint32_t(r[R_ASTR + agent]) << 24);
         sc1 = ((r[R_AFLAGS + agent] & AF_CANKICK) ? 1u : 0u) | (alive << 8) | (uint32_t(r[R_TIME]) << 16) | (uint32_t(r[R_TIME + 1]) << 24);
         sc2 = (alive >> agent) & 1u;
+        if(RADIO) sc2 |= radio_obs_bytes(r, agent);
     }
     POM_LOOP
     for(uint32_t q = uint32_t(i); q < nchunks; q += 4u)
@@ -1941,10 +1980,11 @@ POM_HD void observe_cropped_part_patches(const uint8_t* r, int agent, int view, 
 }
 
 /* the four parts one after the other (tests/hostsim; not used by the kernels) */
+template<bool RADIO = false>
 POM_HD void observe_cropped(const uint8_t* r, int agent, int view, uint8_t* out)
 {
     uint32_t fl[4];
-    for(int i = 0; i < 4; i++) fl[i] = observe_cropped_part_chunks(r, agent, view, out, i);
+    for(int i = 0; i < 4; i++) fl[i] = observe_cropped_part_chunks<RADIO>(r, agent, view, out, i);
     for(int i = 0; i < 4; i++) observe_cropped_part_patches(r, agent, view, out, i, fl[i]);
 }
 

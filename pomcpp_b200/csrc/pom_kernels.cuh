@@ -16,6 +16,7 @@
  *  K4 k_gather_records / k_expand_step           state copy (pom_batch_clone) and tree-search fan-out (+ one Step, fused).
  *  K5 k_pack / k_unpack / k_observe              AoS bboard::State <-> packed record; the State as one agent sees it (fog).
  *     k_observe_planes                            the same view as byte planes for a network input, four lanes per env.
+ *     k_radio_download / k_radio_upload           the team radio's last messages (record bytes 289..291) <-> host words.
  *  K7 k_policy_moves / k_rollout<TPB, true>   the reference's SimpleAgent (pom_policy.cuh) as the action source: per tick
  *                                                 into a moves buffer, or inside the fused rollout; the agents' 8-byte
  *                                                 memories live in global memory, word-major (coalesced, L1/L2-resident).
@@ -356,6 +357,8 @@ __device__ __forceinline__ void warp_tick(uint8_t* sslice, uint8_t* rec, uint32_
  * (pomcore::observe_part_chunks), so that every store instruction of the warp covers eight full 128-byte lines.
  * `out0` = the observation of the slice's first env, `n_valid` = envs of the slice inside the batch.  All 32 lanes call. */
 /* the cropped layout (pomcore::observe_cropped_part_*): records of `rec_bytes`; every lane patches its own flame cells */
+/* RADIO (both forms): the observation of a radio handle, with the teammate's last message (pomcore::radio_obs_bytes) */
+template<bool RADIO = false>
 __device__ __forceinline__ void warp_observe_slice_cropped(const uint8_t* sslice, int agent, int view, uint8_t* out0, uint32_t n_valid, uint32_t rec_bytes)
 {
     const uint32_t lane = threadIdx.x & 31u, quad = lane >> 2;
@@ -368,12 +371,13 @@ __device__ __forceinline__ void warp_observe_slice_cropped(const uint8_t* sslice
         const uint8_t* r = sslice + e * POM_REC_BYTES;
         uint8_t* out = out0 + size_t(e) * rec_bytes;
         uint32_t flames = 0u;
-        if(valid) flames = pomcore::observe_cropped_part_chunks(r, agent, view, out, part);
+        if(valid) flames = pomcore::observe_cropped_part_chunks<RADIO>(r, agent, view, out, part);
         __syncwarp();                                         /* the quad's chunk stores are ordered before its patches */
         if(valid) pomcore::observe_cropped_part_patches(r, agent, view, out, part, flames);
     }
 }
 
+template<bool RADIO = false>
 __device__ __forceinline__ void warp_observe_slice(const uint8_t* sslice, int agent, int view, uint8_t* out0, uint32_t n_valid)
 {
     const uint32_t lane = threadIdx.x & 31u, quad = lane >> 2;
@@ -390,7 +394,7 @@ __device__ __forceinline__ void warp_observe_slice(const uint8_t* sslice, int ag
         if(valid)
         {
             W = pomcore::obs_window(r, agent, view);
-            lit = pomcore::observe_part_chunks(r, agent, W, out, part);
+            lit = pomcore::observe_part_chunks<RADIO>(r, agent, W, out, part);
         }
         lit |= __shfl_xor_sync(FULL_WARP, lit, 1);
         lit |= __shfl_xor_sync(FULL_WARP, lit, 2);
@@ -485,7 +489,8 @@ struct StepIO {
     uint8_t*    status_out;    /* one end-of-tick status byte per env, or null */
     uint32_t*   done_bits;     /* one word per slice: bit l = env 32 s + l ended an episode this tick, or null */
     uint32_t*   fin_env;       /* compacted list of those envs ...            (null: no list) */
-    uint8_t*    fin_status;    /* ... and their status bytes (as in status_out) */
+    uint8_t*    fin_status;    /* ... and their status bytes (as in status_out).  The RADIO images, which keep no list, take
+                                  the caller's messages here: one word per env, byte a = agent a's (pom_batch_step_radio) */
     uint32_t*   fin_counter;   /* DEVICE words: [0] the counter the list is appended through, [1] CTAs that are done */
     uint32_t*   fin_count_out; /* where the last CTA publishes the list length (device or mapped host memory) */
     uint32_t    fin_capacity;
@@ -494,7 +499,8 @@ struct StepIO {
                                   obs + k * obs_stride * POM_OBS_BYTES; null = none.
                                   The REWARDS images, which are OBS = false images, take their output here instead:
                                   one word per env, byte a = the int8 reward of agent a (pomcore::tick_rewards).  The slot
-                                  keeps its one type: a union with a uint32_t* changed the SASS of the OBS images. */
+                                  keeps its one type: a union with a uint32_t* changed the SASS of the OBS images.
+                                  The RADIO images (REWARDS images with a null check) may leave it null. */
     uint64_t    obs_stride;
     uint32_t    obs_mask;
     int         obs_view;
@@ -539,7 +545,12 @@ template<int NBUF> struct RingScratch {
 /* REWARDS: the image of pom_batch_step_rewards - every active env also stores its four int8 rewards (pomcore::tick_rewards)
  * as one word to the array in StepIO::obs, next to its status byte.  Its own image for the reason FREEZE and TEAMS have theirs:
  * the plain step keeps its code as it is. */
-template<int NW, int NBUF, bool OBS, bool FREEZE, bool SPEC = false, bool TEAMS = false, bool REWARDS = false>
+/* RADIO: the image of pom_batch_step_radio (team game only, with REWARDS) - every env that is stepped latches the caller's
+ * four message bytes (StepIO::fin_status, one word per env, fetched with a per-lane load issued before the slice's wait)
+ * into its record's radio bytes before the tick (pomcore::radio_latch).  The rewards pointer may be null here: one image
+ * with a run-time test instead of two, since the test is one predicated store per env and the kernel is bound by HBM.
+ * No done bits, no finished-env list: their slots are forced to null, which keeps fin_status free for the messages. */
+template<int NW, int NBUF, bool OBS, bool FREEZE, bool SPEC = false, bool TEAMS = false, bool REWARDS = false, bool RADIO = false>
 __global__ void __launch_bounds__((NW + 1) * 32, 1) k_step_ws(BatchParams P, StepIO io_in, uint32_t flags_in)
 {
     const uint32_t flags = SPEC ? uint32_t(POM_STEP_AUTORESET | POM_STEP_COUNT) : flags_in;
@@ -547,6 +558,10 @@ __global__ void __launch_bounds__((NW + 1) * 32, 1) k_step_ws(BatchParams P, Ste
     if(SPEC)
     {
         io.joint = 0u; io.bulk = 1u; io.status_out = nullptr; io.obs = nullptr; io.done_bits = nullptr; io.fin_env = nullptr;
+    }
+    if(RADIO)
+    {
+        io.done_bits = nullptr; io.fin_env = nullptr;
     }
     const uint32_t* __restrict__ moves = static_cast<const uint32_t*>(io.moves);
     const uint16_t* __restrict__ joint = static_cast<const uint16_t*>(io.moves);
@@ -621,6 +636,7 @@ __global__ void __launch_bounds__((NW + 1) * 32, 1) k_step_ws(BatchParams P, Ste
         uint32_t m = 0u;
         if(!(moves_bulk && whole) && active) m = io.joint ? uint32_t(__ldg(joint + env)) : __ldg(moves + env);   /* overlaps the wait below */
         uint32_t ep_now = (active && (flags & POM_STEP_AUTORESET)) ? P.episodes[env] : 0u;
+        const uint32_t msg = (RADIO && active) ? __ldg(reinterpret_cast<const uint32_t*>(io.fin_status) + env) : 0u;
         /* where is my slice?  (The mail slot of ticket t is rewritten for ticket t + 256; by then this warp has long read
          * it: the producer is never more than the 24 buffers ahead of the warps.) */
         uint32_t v;
@@ -639,6 +655,7 @@ __global__ void __launch_bounds__((NW + 1) * 32, 1) k_step_ws(BatchParams P, Ste
          * compile-time constant per branch of `raw`.  tools/ab keeps the builds of that A/B.) */
         const bool stepped = active && !(rec[R_STATUS] & ((raw ? POM_STATUS_INVALID : (POM_STATUS_DONE | POM_STATUS_INVALID)) |
                                                           (FREEZE ? POM_STATUS_TRUNCATED : 0)));
+        if(RADIO && stepped) pomcore::radio_latch(rec, msg);
         warp_tick<TEAMS>(sslice, rec, m, stepped, raw, sslice + R::SLICE_BYTES + 128u,
                          (flags & POM_STEP_CONTINUE_UNDEFINED) ? pomcore::F_INVALID_MASK_CONTINUE : pomcore::F_INVALID_MASK);
         acc.steps += stepped ? 1u : 0u;
@@ -650,7 +667,7 @@ __global__ void __launch_bounds__((NW + 1) * 32, 1) k_step_ws(BatchParams P, Ste
         }
         if(status_out && active) status_out[env] = uint8_t(st_end);
         /* after a reset the record is the template's, but tick_rewards reads the agent flags only while the game runs */
-        if(REWARDS && active)
+        if(REWARDS && active && (!RADIO || io.obs))
             reinterpret_cast<uint32_t*>(io.obs)[env] = pomcore::tick_rewards<TEAMS>(stepped, st_end, *reinterpret_cast<const uint32_t*>(rec + R_AFLAGS));
         if(io.done_bits || io.fin_env)
         {
@@ -989,6 +1006,31 @@ __global__ void k_fill_from_templates(BatchParams P)
     reinterpret_cast<uint32_t*>(P.recs)[t] = __ldg(reinterpret_cast<const uint32_t*>(P.templates) + k * POM_REC_WORDS + w);
 }
 
+/* the radio bytes of envs [first, first + count) <-> one word per env in the pom_batch_step_radio encoding (byte a =
+ * agent a's w0 | w1 << 3); the upload ignores bits 6..7 of each byte */
+__global__ void k_radio_download(const uint8_t* __restrict__ recs, uint32_t* __restrict__ out, uint64_t first, uint64_t count)
+{
+    const uint64_t i = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+    if(i >= count) return;
+    const uint8_t* r = recs + (first + i) * POM_REC_BYTES;
+    uint32_t w = 0u;
+    for(int a = 0; a < 4; a++) w |= pomcore::radio_message(r, a) << (8 * a);
+    out[i] = w;
+}
+
+__global__ void k_radio_upload(uint8_t* __restrict__ recs, const uint32_t* __restrict__ in, uint64_t first, uint64_t count)
+{
+    const uint64_t i = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+    if(i >= count) return;
+    uint8_t* r = recs + (first + i) * POM_REC_BYTES;
+    const uint32_t m = in[i];
+    uint32_t v = 0u;
+    for(int a = 0; a < 4; a++) v |= ((m >> (8 * a)) & 63u) << (6 * a);
+    r[R_RADIO] = uint8_t(v);
+    r[R_RADIO + 1] = uint8_t(v >> 8);
+    r[R_RADIO + 2] = uint8_t(v >> 16);
+}
+
 /* ---------------------------------------------------------------- K4: tree-search expansion */
 /* child c = root_i * fanout + j: copy the root's record into the tile, apply joint action j
  * (a_k = (j / 6^k) % 6), Step once, bulk-store the tile.
@@ -1112,7 +1154,8 @@ __global__ void k_observe(const uint8_t* __restrict__ recs, pom_state* aos, uint
  * per env store whole lines.  The fused form is StepIO::obs. */
 /* CROPPED: the image for the cropped layout (with both layouts in one image the kernel needed 127 registers and the full
  * layout lost a third of its speed) */
-template<int TPB, bool CROPPED = false>
+/* RADIO: the images of radio handles (warp_observe_slice<RADIO>) */
+template<int TPB, bool CROPPED = false, bool RADIO = false>
 __global__ void __launch_bounds__(TPB, CROPPED ? 768 / TPB : 0) k_observe_planes(BatchParams P, uint8_t* __restrict__ out, uint64_t stride, uint32_t mask, int view,
                                                                   uint32_t reverse, uint32_t cropped_bytes)
 {
@@ -1140,8 +1183,8 @@ __global__ void __launch_bounds__(TPB, CROPPED ? 768 / TPB : 0) k_observe_planes
     for(int a = 0; a < 4; a++)
     {
         if(!((mask >> a) & 1u)) continue;
-        if(CROPPED) warp_observe_slice_cropped(sslice, a, view, out + (uint64_t(k) * stride + env0) * cropped_bytes, n_valid, cropped_bytes);
-        else warp_observe_slice(sslice, a, view, out + (uint64_t(k) * stride + env0) * POM_OBS_BYTES, n_valid);
+        if(CROPPED) warp_observe_slice_cropped<RADIO>(sslice, a, view, out + (uint64_t(k) * stride + env0) * cropped_bytes, n_valid, cropped_bytes);
+        else warp_observe_slice<RADIO>(sslice, a, view, out + (uint64_t(k) * stride + env0) * POM_OBS_BYTES, n_valid);
         k++;
     }
 }

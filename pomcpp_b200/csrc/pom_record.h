@@ -4,7 +4,8 @@
  * One env = 292 bytes = 73 32-bit words.  73 is odd, so when the 32 lanes of a warp touch the
  * same field of 32 consecutive records in shared memory they hit 32 different banks.
  * 289 bytes are payload (SURVEY Appendix B, the figure behind the 582 B/env-step roofline
- * accounting); 3 bytes pad the record to a word multiple.
+ * accounting); 3 bytes pad the record to a word multiple.  A radio handle keeps its team messages in
+ * those 3 bytes, so the radio adds no byte to what a kernel moves per env.
  *
  * Replaces the reference's 1004-byte AoS `bboard::State` (include/bboard.hpp:356-383).
  *
@@ -27,7 +28,8 @@
  *  248     20     flames.queue[20].timeLeft (signed byte)
  *  268     20     flames.queue[20].strength
  *  288     1      flames.index
- *  289     3      padding (zero)
+ *  289     3      radio (handles made with POM_INIT_RADIO), zero otherwise: the last message of agent a, w0 | w1 << 3
+ *                 (two 3-bit words), in bits 6a..6a+5 of the little-endian 24-bit value (pomcore::radio_latch)
  *
  * Cell codes (1 byte, bijective on every value the reference can produce, bboard.hpp:54-71):
  *   0 PASSAGE  1 RIGID  2..6 WOOD+flag(0..4)  7 BOMB  8 FOG  9 EXTRABOMB  10 INCRRANGE  11 KICK
@@ -64,7 +66,8 @@ enum {
     R_FPOS   = 228,
     R_FTIME  = 248,
     R_FSTR   = 268,
-    R_FINDEX = 288
+    R_FINDEX = 288,
+    R_RADIO  = 289
 };
 
 enum {

@@ -307,8 +307,8 @@ Move Environment::GetLastMove(int agentID) { return lastMoves[agentID]; }
 
 /* ---- BatchEnvironment ---- */
 BatchEnvironment::BatchEnvironment(size_t nGames, int device, uint64_t envOffset, uint32_t nTemplates, int firstSeed, uint32_t maxTicks,
-                                   bool teams)
-    : n(nGames), teams(teams)
+                                   bool teams, bool radio)
+    : n(nGames), teams(teams), radio(radio)
 {
     pom_init_desc d;
     std::memset(&d, 0, sizeof(d));
@@ -316,7 +316,7 @@ BatchEnvironment::BatchEnvironment(size_t nGames, int device, uint64_t envOffset
     d.n_templates = nTemplates;
     d.first_seed = firstSeed;
     d.max_ticks = maxTicks;
-    d.flags = teams ? POM_INIT_TEAMS : 0;
+    d.flags = (teams ? POM_INIT_TEAMS : 0) | (radio ? POM_INIT_RADIO : 0);
     check(pom_batch_init(&handle, device, n, &d), "pom_batch_init");
     movebuf.resize(4 * n);
 }
@@ -414,6 +414,41 @@ size_t BatchEnvironment::Step(const Move* moves, int8_t* rewards)
     size_t running = 0;
     for(size_t i = 0; i < n; i++) running += (status[i] & (POM_STATUS_DONE | POM_STATUS_INVALID)) ? 0 : 1;
     return running;
+}
+
+size_t BatchEnvironment::StepRadio(const Move* moves, const uint8_t* messages, int8_t* rewards)
+{
+    /* one pinned buffer the kernel reads and writes directly: moves, messages, rewards, status bytes */
+    void* pinned = nullptr;
+    check(pom_host_alloc(13 * n, &pinned), "pom_host_alloc");
+    uint8_t* mv = static_cast<uint8_t*>(pinned);
+    uint8_t* msg = mv + 4 * n;
+    int8_t* rw = reinterpret_cast<int8_t*>(mv + 8 * n);
+    uint8_t* st = mv + 12 * n;
+    for(size_t i = 0; i < 4 * n; i++) mv[i] = uint8_t(int(moves[i]));
+    std::memcpy(msg, messages, 4 * n);
+    int rc = pom_batch_step_radio(handle, mv, msg, 0, rewards ? rw : nullptr, st);
+    if(rc == POM_OK) rc = pom_batch_sync(handle);
+    if(rc == POM_OK)
+    {
+        if(rewards) std::memcpy(rewards, rw, 4 * n);
+        status.assign(st, st + n);
+    }
+    pom_host_free(pinned);
+    check(rc, "pom_batch_step_radio");
+    fresh = false;
+    tick++;
+    size_t running = 0;
+    for(size_t i = 0; i < n; i++) running += (status[i] & (POM_STATUS_DONE | POM_STATUS_INVALID)) ? 0 : 1;
+    return running;
+}
+
+std::pair<int, int> BatchEnvironment::GetMessage(size_t i, int agent)
+{
+    uint8_t m[4];
+    check(pom_batch_radio_download(handle, i, 1, m), "pom_batch_radio_download");
+    const int v = m[agent & 3];
+    return std::make_pair(v & 7, v >> 3);
 }
 
 size_t BatchEnvironment::StepSequence(const Move* moves, uint32_t ticks)
