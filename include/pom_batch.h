@@ -123,6 +123,10 @@ const char* pom_last_error(void);
 int  pom_batch_teams(const pom_batch* b);
 /* 1 if the handle has the team radio (POM_INIT_RADIO), 0 if not, POM_E_ARG for a null handle */
 int  pom_batch_radio(const pom_batch* b);
+/* *out = 1 if the handle's record array lives in compressible device memory (granted by the driver where the device
+ * supports generic compression; the array is then rounded up to the allocation granularity), 0 if it came from
+ * cudaMalloc.  A read-only report of what the handle got: results are the same either way. */
+int  pom_batch_records_compressed(const pom_batch* b, int* out);
 
 /* ---- AoS <-> packed exchange (there is no reference call: State is passed by pointer) ---- */
 int  pom_batch_upload(pom_batch* b, uint64_t first, uint64_t count, const pom_state* states, const uint8_t* status /* may be NULL */);

@@ -238,6 +238,15 @@ class Batch:
         _ck(min(r, 0))
         return r == 1
 
+    def records_compressed(self):
+        """True if the record array lives in compressible device memory (pom_batch_records_compressed): a report, not a switch"""
+        # looked up here, not bound in lib(), so that POM_B200_LIB can still load builds that predate it (A/B runs)
+        f = lib().pom_batch_records_compressed
+        f.argtypes = [C.c_void_p, C.POINTER(C.c_int)]
+        v = C.c_int()
+        _ck(f(self.h, C.byref(v)))
+        return v.value == 1
+
     def radio_download(self, first=0, count=None):
         """[count, 4] uint8: every env's last message per agent, byte a = w0 | w1 << 3 (unpack_messages splits it)"""
         count = self.n - first if count is None else count

@@ -5,6 +5,8 @@
  * in the sm_100a kernels of pom_kernels.cuh.  There is deliberately no host stepping path here:
  * without a CUDA device every entry point fails with POM_E_CUDA.
  */
+#include <cuda.h>
+#include <cudaTypedefs.h>
 #include <cuda_runtime.h>
 #include <cstdio>
 #include <cstdlib>
@@ -44,6 +46,124 @@ struct DevBuf {
 
 #define CK(expr) do { cudaError_t ce_ = (expr); if(ce_ != cudaSuccess) return fail(POM_E_CUDA, #expr, ce_); } while(0)
 
+/* The record array in compressible device memory.  Each tick streams the whole array through DRAM, and most of a
+ * record's bytes are zero (empty board cells, unused bomb and flame ring slots, the pad bytes): with generic compression
+ * the hardware moves fewer DRAM bytes for the same lines, losslessly and unseen by the kernels.  Compressible memory
+ * exists only through the driver's virtual memory API; its entry points are looked up at run time, so the library
+ * links against the runtime alone. */
+struct Driver {
+    PFN_cuDeviceGet_v2000 DeviceGet = nullptr;
+    PFN_cuDeviceGetAttribute_v2000 DeviceGetAttribute = nullptr;
+    PFN_cuMemGetAllocationGranularity_v10020 MemGetAllocationGranularity = nullptr;
+    PFN_cuMemCreate_v10020 MemCreate = nullptr;
+    PFN_cuMemGetAllocationPropertiesFromHandle_v10020 MemGetAllocationPropertiesFromHandle = nullptr;
+    PFN_cuMemAddressReserve_v10020 MemAddressReserve = nullptr;
+    PFN_cuMemMap_v10020 MemMap = nullptr;
+    PFN_cuMemSetAccess_v10020 MemSetAccess = nullptr;
+    PFN_cuMemUnmap_v10020 MemUnmap = nullptr;
+    PFN_cuMemRelease_v10020 MemRelease = nullptr;
+    PFN_cuMemAddressFree_v10020 MemAddressFree = nullptr;
+    bool ok = false;
+};
+
+template<typename F>
+bool entry(const char* name, F* fn)
+{
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+    if(cudaGetDriverEntryPointByVersion(name, &p, 12000, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess || !p)
+    {
+        cudaGetLastError();
+        return false;
+    }
+    *fn = reinterpret_cast<F>(p);
+    return true;
+}
+
+const Driver& driver()
+{
+    static const Driver d = [] {
+        Driver x;
+        x.ok = entry("cuDeviceGet", &x.DeviceGet) && entry("cuDeviceGetAttribute", &x.DeviceGetAttribute) &&
+               entry("cuMemGetAllocationGranularity", &x.MemGetAllocationGranularity) && entry("cuMemCreate", &x.MemCreate) &&
+               entry("cuMemGetAllocationPropertiesFromHandle", &x.MemGetAllocationPropertiesFromHandle) &&
+               entry("cuMemAddressReserve", &x.MemAddressReserve) && entry("cuMemMap", &x.MemMap) &&
+               entry("cuMemSetAccess", &x.MemSetAccess) && entry("cuMemUnmap", &x.MemUnmap) &&
+               entry("cuMemRelease", &x.MemRelease) && entry("cuMemAddressFree", &x.MemAddressFree);
+        return x;
+    }();
+    return d;
+}
+
+/* Maps `bytes` (rounded up to the allocation granularity) of compressible memory on `device`; returns the mapped size, or
+ * 0 when the device, the driver or the grant says no.  The driver may hand out uncompressible memory for a compressible
+ * request: the granted properties are read back and such memory is given back. */
+size_t map_compressible(int device, size_t bytes, void** out)
+{
+    const Driver& d = driver();
+    if(!d.ok) return 0;
+    CUdevice dev = 0;
+    int vmm = 0, comp = 0;
+    if(d.DeviceGet(&dev, device) != CUDA_SUCCESS ||
+       d.DeviceGetAttribute(&vmm, CU_DEVICE_ATTRIBUTE_VIRTUAL_MEMORY_MANAGEMENT_SUPPORTED, dev) != CUDA_SUCCESS || !vmm ||
+       d.DeviceGetAttribute(&comp, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, dev) != CUDA_SUCCESS || !comp)
+        return 0;
+    CUmemAllocationProp prop = {};
+    prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop.location.id = dev;
+    prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+    size_t gran = 0;
+    if(d.MemGetAllocationGranularity(&gran, &prop, CU_MEM_ALLOC_GRANULARITY_MINIMUM) != CUDA_SUCCESS || gran == 0) return 0;
+    const size_t size = (bytes + gran - 1) / gran * gran;
+    CUmemGenericAllocationHandle h = 0;
+    if(d.MemCreate(&h, size, &prop, 0) != CUDA_SUCCESS) return 0;
+    CUmemAllocationProp got = {};
+    CUdeviceptr va = 0;
+    CUmemAccessDesc access = {};
+    access.location = prop.location;
+    access.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+    const bool granted = d.MemGetAllocationPropertiesFromHandle(&got, h) == CUDA_SUCCESS &&
+                         got.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_GENERIC;
+    const bool reserved = granted && d.MemAddressReserve(&va, size, gran, 0, 0) == CUDA_SUCCESS;
+    const bool mapped = reserved && d.MemMap(va, size, 0, h, 0) == CUDA_SUCCESS;
+    const bool ok = mapped && d.MemSetAccess(va, size, &access, 1) == CUDA_SUCCESS;
+    d.MemRelease(h);                           /* from here on the mapping alone holds the memory */
+    if(!ok)
+    {
+        if(mapped) d.MemUnmap(va, size);
+        if(reserved) d.MemAddressFree(va, size);
+        return 0;
+    }
+    *out = reinterpret_cast<void*>(va);
+    return size;
+}
+
+/* the handle's record array: compressible memory where the device grants it, cudaMalloc otherwise.  *mapped is the
+ * compressible mapping's size, 0 for cudaMalloc: it selects how free_records gives the memory back.
+ * Only the records: pom_device_alloc (the bench's move ring, observation slabs) and the template pool in compressible
+ * memory as well measured within 0.1 % of this on every leg of bench.py (B200, profiles/bench_compressible.jsonl), so
+ * they stay on cudaMalloc. */
+cudaError_t alloc_records(int device, size_t bytes, uint8_t** out, size_t* mapped)
+{
+    void* p = nullptr;
+    *mapped = map_compressible(device, bytes, &p);
+    if(*mapped) { *out = static_cast<uint8_t*>(p); return cudaSuccess; }
+    return cudaMalloc(reinterpret_cast<void**>(out), bytes);
+}
+
+void free_records(uint8_t* p, size_t mapped)
+{
+    if(!p) return;
+    if(!mapped) { cudaFree(p); return; }
+    /* cudaFree waits for the device before it frees; an unmap is given the same wait, so that no kernel of any handle
+     * on this device (an expansion reading these records into another handle) still uses the range */
+    cudaDeviceSynchronize();
+    const Driver& d = driver();
+    d.MemUnmap(reinterpret_cast<CUdeviceptr>(p), mapped);
+    d.MemAddressFree(reinterpret_cast<CUdeviceptr>(p), mapped);
+}
+
 constexpr uint64_t TILE_ALIGN = 256;           /* records are allocated in whole tiles of the largest TPB */
 constexpr uint64_t XFER_CHUNK = 65536;         /* envs per AoS staging chunk (66 MB)                      */
 constexpr size_t   FLUSH_BYTES = size_t(256) << 20;
@@ -75,6 +195,7 @@ struct pom_batch {
     int       policy_view = -1;                /* pom_batch_set_policy_view: >= 0 = the device SimpleAgent plays under fog of war
                                                   with this view (the FOG images, POM_DISPATCH_POLICY), < 0 = on the full state */
     uint8_t*  recs = nullptr;
+    size_t    recs_mapped = 0;                 /* bytes of compressible memory mapped for recs (alloc_records); 0 = cudaMalloc */
     uint8_t*  templates = nullptr;
     uint32_t* episodes = nullptr;
     unsigned long long* stats = nullptr;
@@ -551,7 +672,7 @@ int pom_batch_init(pom_batch** out, int device, uint64_t n_envs, const pom_init_
            cudaEventCreateWithFlags(&b->ev_out, cudaEventDisableTiming) != cudaSuccess ||
            cudaEventCreateWithFlags(&b->ev_begin, cudaEventDisableTiming) != cudaSuccess)
         { rc = fail(POM_E_CUDA, "stream/event creation failed", cudaGetLastError()); break; }
-        if(cudaMalloc(&b->recs, b->n_alloc * POM_REC_BYTES) != cudaSuccess ||
+        if(alloc_records(device, b->n_alloc * POM_REC_BYTES, &b->recs, &b->recs_mapped) != cudaSuccess ||
            cudaMalloc(&b->templates, size_t(b->n_templates) * POM_REC_BYTES) != cudaSuccess ||
            cudaMalloc(&b->episodes, b->n_alloc * sizeof(uint32_t)) != cudaSuccess ||
            cudaMalloc(&b->stats, POM_STATS_WORDS * sizeof(unsigned long long)) != cudaSuccess ||
@@ -592,7 +713,7 @@ int pom_batch_destroy(pom_batch* b)
     cudaSetDevice(b->device);
     if(b->s_k2) cudaStreamSynchronize(b->s_k2);
     if(b->stream) cudaStreamSynchronize(b->stream);
-    cudaFree(b->recs); cudaFree(b->templates); cudaFree(b->episodes); cudaFree(b->stats);
+    free_records(b->recs, b->recs_mapped); cudaFree(b->templates); cudaFree(b->episodes); cudaFree(b->stats);
     cudaFree(b->moves_buf); cudaFree(b->status_buf); cudaFree(b->aos_stage); cudaFree(b->st_stage);
     cudaFree(b->bad_count); cudaFree(b->flush_buf); cudaFree(b->idx_buf); if(b->ev_expand) cudaEventDestroy(b->ev_expand); cudaFree(b->policy); cudaFree(b->fin_counter);
     if(b->ev[0]) cudaEventDestroy(b->ev[0]);
@@ -1252,6 +1373,13 @@ int pom_batch_generate_moves(pom_batch* b, uint8_t* moves_dev, uint64_t seed, ui
 uint64_t pom_batch_size(const pom_batch* b) { return b ? b->n_envs : 0; }
 int      pom_batch_teams(const pom_batch* b) { return b ? (b->teams ? 1 : 0) : fail(POM_E_ARG, "pom_batch_teams: null handle"); }
 int      pom_batch_radio(const pom_batch* b) { return b ? (b->radio ? 1 : 0) : fail(POM_E_ARG, "pom_batch_radio: null handle"); }
+
+int pom_batch_records_compressed(const pom_batch* b, int* out)
+{
+    if(!b || !out) return fail(POM_E_ARG, "pom_batch_records_compressed: null argument");
+    *out = b->recs_mapped != 0;
+    return POM_OK;
+}
 
 int pom_batch_radio_download(pom_batch* b, uint64_t first, uint64_t count, uint8_t* msgs_host)
 {
