@@ -81,7 +81,9 @@ typedef struct pom_init_desc {
                                          are free of the reference's uninitialised-read defect (bboard.cpp:351,367,372),
                                          generated ON THE DEVICE (mt19937_64 + libstdc++ uniform_int_distribution)   */
     const pom_state* host_templates;  /* if non-NULL: n_templates AoS states to use as the pool instead             */
-    uint32_t         max_ticks;       /* rollout truncation (Pommerman: 800); 0 = never                      */
+    uint32_t         max_ticks;       /* rollout truncation (Pommerman: 800); 0 = never.  timeStep is 16 bits on the
+                                         device, so values above 65535 never truncate: an env that plays on is aborted
+                                         as POM_STATUS_INVALID on its 65 536th tick instead (timeStep stays 65535) */
     uint32_t         flags;           /* POM_INIT_*                                                            */
 } pom_init_desc;
 
@@ -109,7 +111,9 @@ typedef struct pom_stats {
     uint64_t truncated;        /* timeStep reached max_ticks                         */
     uint64_t sum_episode_len;  /* sum of timeStep over finished episodes             */
     uint64_t invalid;          /* episodes aborted because the env left the reference's defined domain
-                                  (the reference itself would crash or hang there, SURVEY §8c D3-D5)  */
+                                  (the reference itself would crash or hang there, SURVEY §8c D3-D5), or
+                                  because it reached the 16-bit timeStep ceiling (see max_ticks).  An episode that
+                                  ends DONE or TRUNCATED in that same tick counts there, not here */
 } pom_stats;
 #define POM_STATS_WORDS 10
 

@@ -120,7 +120,13 @@ __device__ __forceinline__ void warp_add(unsigned long long* dst, uint32_t v)
 /* Episode statistics are gathered per lane in registers (16-bit counters, two to a word) and added to the global
  * counters ONCE per warp and launch (acc_flush): one warp reduction and one atomicAdd per counter, instead of three
  * reductions and up to nine atomics in every tick in which some env of the warp finished (1.3 M warp-instructions per
- * 1 Mi-env tick, profiles/k_step_by_function_r2.txt). */
+ * 1 Mi-env tick, profiles/k_step_by_function_r2.txt).
+ * Width: a lane counts at most one finished episode per tick in k_rollout, which flushes every 16383 ticks; k_step_ws
+ * flushes once per launch, and a lane counts at most one finish per slice its warp takes.  Warps take slices by ticket,
+ * so one warp could in principle take all ceil(n_slices / grid) slices of its CTA; on average a lane sees
+ * n / (SMs x 20 x 32) envs: 11 at 1 Mi envs, about 6 300 at the ~600 M envs that 180 GB of HBM hold.  A counter can
+ * only wrap above ~310 M envs per handle (65 536 slices per CTA), and then only if one warp takes more than half of
+ * its CTA's slices. */
 struct EpisodeAcc {
     uint32_t fin_draw = 0u;      /* episodes | draws << 16      */
     uint32_t trunc_abort = 0u;   /* truncated | aborted << 16   */
