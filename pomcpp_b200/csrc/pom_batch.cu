@@ -188,6 +188,9 @@ struct pom_batch {
     int       obs_fused = 0;                   /* POM_OBS_FUSED=1: pom_batch_step_observe / pom_step_compact_io::obs_dev write the planes
                                                   from inside the step kernel instead of launching k_observe_planes behind it */
     int       step_kernel = 0;                 /* 0 = k_step_ws (persistent, warp-specialised), 1 = k_step (one CTA per tile); POM_STEP_KERNEL=tile */
+    int       step_parts = 2;                  /* POM_STEP_PARTS=2..16: launches per pom_batch_step with POM_STEP_OVERLAP */
+    int       chunks = 6;                      /* POM_CHUNKS=1..MAX_CHUNKS: chunks of pom_batch_step_host's copy pipeline */
+    int       zerocopy = 1;                    /* POM_ZEROCOPY=0: pom_batch_step_host takes the copy pipeline for pinned buffers too */
     bool      teams = false;                   /* POM_INIT_TEAMS: the 2v2 team game, fixed for the handle's life; every stepping or
                                                   acting launch takes the kernel images of this mode (POM_DISPATCH_MODE) */
     bool      radio = false;                   /* POM_INIT_RADIO (team game only, fixed for the handle's life): the records' radio bytes
@@ -661,6 +664,17 @@ int pom_batch_init(pom_batch** out, int device, uint64_t n_envs, const pom_init_
         const int t = std::atoi(e);
         if(t == 32 || t == 64 || t == 128 || t == 256) b->tpb = t;
     }
+    if(const char* e = std::getenv("POM_STEP_PARTS"))
+    {
+        const int p = std::atoi(e);
+        if(p >= 2 && p <= 16) b->step_parts = p;
+    }
+    if(const char* e = std::getenv("POM_CHUNKS"))
+    {
+        const int c = std::atoi(e);
+        if(c >= 1 && c <= pom_batch::MAX_CHUNKS) b->chunks = c;
+    }
+    if(const char* e = std::getenv("POM_ZEROCOPY")) b->zerocopy = std::atoi(e);
     int rc = POM_OK;
     do {
         if(cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking) != cudaSuccess ||
@@ -845,8 +859,7 @@ int pom_batch_step(pom_batch* b, const uint8_t* moves_dev, uint32_t flags)
      * caller's moves, the first half of the previous tick) and, by stream order, for its own previous tick; the first
      * half of the NEXT tick does not wait for it.  So the last, partly filled wave of one kernel runs next to the first
      * wave of the other, tick after tick; use() joins the streams before any other operation. */
-    static int parts = -1;
-    if(parts < 0) { const char* e = std::getenv("POM_STEP_PARTS"); parts = e ? std::atoi(e) : 2; if(parts < 2 || parts > 16) parts = 2; }
+    const int parts = b->step_parts;
     const uint64_t per = ((b->n_envs + parts - 1) / parts + 1023) / 1024 * 1024;
     /* Up to 0.5 Mi envs the two parts run on the tile kernel: its small CTAs let the two launches share every SM (the
      * persistent kernel takes a whole SM per CTA, so its two launches can only follow each other), and with 60 slices or
@@ -935,9 +948,7 @@ int pom_batch_step_host(pom_batch* b, const uint8_t* moves_host, uint8_t* status
     /* Pinned (page-locked, mapped) host buffers: the kernel reads the move bytes from and writes the status bytes to host
      * memory itself (its one coalesced load per warp is issued before the wait for the bulk state copy, so the PCIe
      * latency hides behind it); no staging copies, no chunks.  POM_ZEROCOPY=0 forces the copy pipeline. */
-    static int zerocopy = -1;
-    if(zerocopy < 0) { const char* e = std::getenv("POM_ZEROCOPY"); zerocopy = e ? std::atoi(e) : 1; }
-    if(zerocopy)
+    if(b->zerocopy)
     {
         rc = launch_step_zero_copy(b, moves_host, status_host, flags);
         if(rc < 0) return rc;
@@ -951,9 +962,7 @@ int pom_batch_step_host(pom_batch* b, const uint8_t* moves_host, uint8_t* status
     /* Pageable buffers: staged copies.  POM_CHUNKS is a tuning knob for experiments; the default is the measured best for 1 Mi envs (6 chunks on two
      * compute streams: 175 us per tick against 219 us for 3 chunks on one stream; submitting the same pipeline as a
      * CUDA graph was measured too and is slower than the direct calls, 182 us) */
-    static int want = -1;
-    if(want < 0) { const char* e = std::getenv("POM_CHUNKS"); want = e ? std::atoi(e) : 6; if(want < 1 || want > pom_batch::MAX_CHUNKS) want = 6; }
-    int chunks = n >= (uint64_t(1) << 18) ? want : 1;
+    int chunks = n >= (uint64_t(1) << 18) ? b->chunks : 1;
     const uint64_t per = ((n + chunks - 1) / chunks + 1023) / 1024 * 1024;      /* multiple of every TPB */
     chunks = int((n + per - 1) / per);
     for(int c = 0; c < chunks; c++)
